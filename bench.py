@@ -4,6 +4,7 @@
   python bench.py [--gpus N --steps K --warmup W]            our arm (CUDA engine), config C4
   python bench.py --impl reference [...]                      the reference's own CPU path, same config
   python bench.py --config C5|C1|C2|C3 [...]                  the other BASELINE.json configurations, same schema
+  python bench.py --dump-outputs DIR [...]                    also write the last timed step's outputs to DIR
 
 Workload at the defaults (BASELINE.json, config C4): synthetic 1024 taxa x 1,000,000 binary site patterns,
 GTR + discrete-Gamma-4, one *step* = one full Felsenstein pruning pass (log-likelihood evaluation) keeping the
@@ -43,7 +44,9 @@ REAL = {   # BASELINE.json configs[0..2]
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps: likelihood evaluations for C4 / C5 (default 20), MCMC generations for C1 - C3 "
+                         "(default 20000 / 4000 / 4000)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="C4", choices=["C4", "C5", "C1", "C2", "C3"])
@@ -51,7 +54,19 @@ def parse():
     ap.add_argument("--patterns", type=int, default=None)
     ap.add_argument("--ref-chunk", type=int, default=12500, help="sites per matML call of --impl reference (divides 125000)")
     ap.add_argument("--no-extras", action="store_true", help="skip cpu_baseline / dirty-path / MCMC extras")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path computed in its last step as DIR/<name>.npy, float64. C4 / C5: "
+                         "lnL.npy and partial_log.npy, the natural log of a fixed, seeded sample of the kept partial "
+                         "cache; C5 on one GPU at the default size keeps no cache and writes lnL.npy only, and with "
+                         "--gpus > 1 the sample is drawn from rank 0's patterns, so compare runs with equal --gpus. "
+                         "C1 - C3: the final state of the chain (lnL, pi, rates, alpha, tree)")
     a = ap.parse_args()
+    if a.steps is not None and a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.steps is None and a.config not in REAL:
+        a.steps = 20
+    if a.dump_outputs is not None and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if a.taxa is None:
         a.taxa = 512 if a.config == "C5" else 1024
     if a.patterns is None:
@@ -179,6 +194,47 @@ class ClockSampler:
                 "samples_whole_run": len(rows), "sm_mhz_min": min((r[1] for r in inside), default=None),
                 "sampler": f"NVML every 5 ms; clocks: {scope}; reasons: warm-up to 150 ms after the timed region (the "
                            "power-cap flag lags the load)"}
+
+
+DUMP_NODES = 16
+DUMP_PARTIAL_BYTES = 48 << 20
+
+
+def dump_outputs(out_dir, eng, snap, lnl, nodes):
+    """--dump-outputs of C4 / C5: what the timed path handed back in its last step, so that two builds can be compared
+    output by output on the same seeded inputs.  lnL.npy holds the log-likelihood (float64, shape (1,)).  When the
+    step keeps the partial cache (snap >= 0), a fixed, seeded sample of it is read back through the snapshot and
+    written as partial_log.npy (DUMP_NODES internal nodes, C, S, patterns): the natural log of each partial
+    likelihood, log(mantissa) + exponent * ln 2, which does not depend on where a build rescales and does not
+    underflow near the root.  The patterns are as many of this rank's as fit in DUMP_PARTIAL_BYTES, so the files
+    stay below 64 MB in all."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "lnL.npy"), np.array([lnl], dtype=np.float64))
+    if snap < 0:
+        return
+    rng = np.random.default_rng(SEED)
+    nodes = np.sort(rng.choice(np.asarray(nodes), size=min(DUMP_NODES, len(nodes)), replace=False))
+    C, S, P = eng.n_cats, eng.n_states, eng.n_patterns
+    n = min(P, DUMP_PARTIAL_BYTES // (len(nodes) * C * S * 8))
+    cols = np.sort(rng.choice(P, size=n, replace=False))
+    out = np.empty((len(nodes), C, S, n))
+    for i, node in enumerate(nodes):
+        m, e = eng.read_partial(snap, int(node), with_scale=True)
+        with np.errstate(divide="ignore"):     # a partial of exactly 0 is written as -inf
+            out[i] = np.log(m[:, :, cols]) + e[cols] * np.log(2.0)
+    np.save(os.path.join(out_dir, "partial_log.npy"), out)
+
+
+def dump_chain_state(out_dir, st):
+    """--dump-outputs of C1 - C3: the state the timed chain ends in, float64: lnL.npy (shape (1,)), pi.npy, rates.npy
+    (exchangeabilities; empty where the model has none), alpha.npy (shape (1,)) and tree.npy, one row (parent, child,
+    branch length) per edge, sorted by (parent, child)."""
+    os.makedirs(out_dir, exist_ok=True)
+    tree = sorted((p, c, t) for (p, c), t in st["tree"].items())
+    rates = np.zeros(0) if st["rates"] is None else st["rates"]
+    for name, v in (("lnL", [st["logLikehood"]]), ("pi", st["pi"]), ("rates", rates), ("alpha", [st["srates"]]),
+                    ("tree", tree)):
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(v, dtype=np.float64))
 
 
 def host_cores():
@@ -434,9 +490,14 @@ def run_c4(a):
     n_e = len(ekeys)
     pi = aln.pi
 
-    def step():
+    kept = []
+
+    def step(keep=False):
         lnl, snap = eng.eval(None, plan.nodes, plan.children, pslots, pi, want_snapshot=True)
-        eng.release_snapshot(snap)
+        if keep:
+            kept.append(snap)
+        else:
+            eng.release_snapshot(snap)
         return lnl
 
     def barrier():
@@ -455,8 +516,8 @@ def run_c4(a):
     eng.host_profile()
     eng.mark(0)
     t0 = time.perf_counter()
-    for _ in range(a.steps):
-        lnl = step()
+    for i in range(a.steps):
+        lnl = step(keep=a.dump_outputs is not None and i == a.steps - 1)
         kernel_ms.append(eng.last_eval_ms())
         main_ms.append(eng.last_eval_main_ms())
     eng.mark(1)
@@ -468,6 +529,10 @@ def run_c4(a):
     info = eng.last_eval_info()
     barrier()
     clock_rec = clocks.stop() if clocks else None
+    if kept:
+        if rank == 0:
+            dump_outputs(a.dump_outputs, eng, kept[0], lnl, plan.nodes[:-1])
+        eng.release_snapshot(kept[0])
     dev_ms, wall_ms = _max_over_ranks(dist, dev_ms, wall * 1e3)
     ms_per_step = dev_ms / a.steps
     value = 1e3 / ms_per_step
@@ -746,9 +811,13 @@ def run_c5(a):
     pi = aln.pi
     keep_cache = (N - 2) * C * S * n_local * 8 <= 150e9
 
-    def step():
+    kept = []
+
+    def step(keep=False):
         lnl, snap = eng.eval(None, plan.nodes, plan.children, pslots, pi, want_snapshot=keep_cache)
-        if snap >= 0:
+        if keep:
+            kept.append(snap)
+        elif snap >= 0:
             eng.release_snapshot(snap)
         return lnl
 
@@ -765,8 +834,8 @@ def run_c5(a):
     st0 = eng.stats()
     kernel_ms, main_ms = [], []
     eng.mark(0)
-    for _ in range(a.steps):
-        lnl = step()
+    for i in range(a.steps):
+        lnl = step(keep=a.dump_outputs is not None and i == a.steps - 1)
         kernel_ms.append(eng.last_eval_ms())
         main_ms.append(eng.last_eval_main_ms())
     eng.mark(1)
@@ -776,6 +845,11 @@ def run_c5(a):
     info = eng.last_eval_info()
     barrier()
     clock_rec = clocks.stop() if clocks else None
+    if kept:
+        if rank == 0:
+            dump_outputs(a.dump_outputs, eng, kept[0], lnl, plan.nodes[:-1])
+        if kept[0] >= 0:
+            eng.release_snapshot(kept[0])
     dev_ms = _max_over_ranks(dist, dev_ms)
     ms_per_step = dev_ms / a.steps
     n_int_edges = sum(1 for (p, c) in ekeys if c > N)
@@ -930,19 +1004,22 @@ def run_real(a):
     wall, dev = wall[a.warmup:], dev[a.warmup:]
     n_states, n_patterns, n_taxa, n_sites = config.N_CHARS, eng.n_patterns, config.N_TAXA, config.N_SITES
     likelihood.reset_engines()
-    n_gen = {"C1": 20000, "C2": 4000, "C3": 4000}[a.config]
+    n_gen = a.steps if a.steps is not None else {"C1": 20000, "C2": 4000, "C3": 4000}[a.config]
     res = run_chain(os.path.join(DATA, fname), model, n_gen, 1000, dtype, os.path.join(tempfile.gettempdir(), "b_" + a.config),
                     reader=reader, out=io.StringIO(), fast_spr=True)
     gens = res["gens_per_sec"]
-    fast = None
+    fast, timed = None, res
     try:
         from cybayes_b200.fastchain import run_chain_native
         likelihood.reset_engines()
         r2 = run_chain_native(os.path.join(DATA, fname), model, n_gen, 1000, dtype,
                               os.path.join(tempfile.gettempdir(), "bn_" + a.config), reader=reader, out=io.StringIO())
         fast = {"gens_per_sec": r2["gens_per_sec"], "same_final_lnL": float(r2["state"]["logLikehood"]) == float(res["state"]["logLikehood"])}
+        timed = r2
     except ImportError:
         pass
+    if a.dump_outputs is not None:
+        dump_chain_state(a.dump_outputs, timed["state"])
     clock_rec = clocks.stop()
     peak, peak_src = measured_peaks()
     req = info_full["bytes_written"] + info_full["bytes_read"]

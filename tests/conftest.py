@@ -65,12 +65,11 @@ def gpu_backend():
 
 
 def run_reference_script(script_name, argv, monkeypatch, capsys):
-    """Run one of the reference's unmodified, byte-compiled driver scripts (oracle/_ref/<name>.code, or
-    the .py under /root/reference when that exists) on top of cybayes_b200/compat; returns its stdout."""
+    """Run one of the reference's unmodified, byte-compiled driver scripts (oracle/_ref/<name>.code, built by
+    oracle/build_ref.sh from a CyBayes checkout; the project does not vendor the reference's code) on top of
+    cybayes_b200/compat; returns its stdout."""
     import runpy
     path = os.path.join(REPO, "oracle", "_ref", script_name + ".code")
-    if not os.path.exists(path):
-        path = os.path.join("/root/reference", script_name + ".py")
     if not os.path.exists(path):
         pytest.skip("no reference driver available (oracle/build_ref.sh)")
     monkeypatch.syspath_prepend(os.path.join(REPO, "cybayes_b200", "compat"))

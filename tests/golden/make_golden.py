@@ -198,7 +198,7 @@ def main():
         json.dump({"generator": "tests/golden/make_golden.py", "cases": cases}, fh, indent=0)
 
 
-if __name__ == "__main__" and not (len(sys.argv) > 1 and sys.argv[1] in ("--nongamma", "--c1-100k")):
+if __name__ == "__main__" and not (len(sys.argv) > 1 and sys.argv[1] in ("--nongamma", "--c1-100k", "--random-inputs")):
     main()
 
 
@@ -285,3 +285,44 @@ def run_c1_100k(n_gen=100000, thin=1000, workdir="/tmp"):
 
 if __name__ == "__main__" and len(sys.argv) > 1 and sys.argv[1] == "--c1-100k":
     run_c1_100k()
+
+
+# ---- seeded random inputs of tests/test_oracle.py: their expected outputs, stored ---------------------------------
+def random_input_vectors(out, source):
+    """Write golden_io.random_vectors of every golden_io.random_inputs case to `out` (.npz), computed by the compiled
+    reference (source "reference": oracle/_ref; run this in a fresh interpreter, its module names are top-level) or by
+    the NumPy oracle (source "oracle"), with a `source` entry naming which."""
+    import numpy as np
+    sys.path.insert(0, os.path.join(REPO, "oracle"))
+    import golden_io
+    import pruning_oracle as oracle
+    if source == "reference":
+        sys.path.insert(0, REF_BUILD)
+        import config, mcmc_gamma, ML_gamma  # the compiled reference
+    rec = {"source": np.array(source)}
+    for i, c in enumerate(golden_io.random_inputs()):
+        tree, root, pi, ll, N, P = c["tree"], c["root"], c["pi"], c["ll"], c["n_taxa"], c["n_sites"]
+        if source == "reference":
+            config.N_TAXA, config.N_CHARS, config.N_SITES, config.MODEL, config.IN_DTYPE = N, c["S"], P, c["model"], c["dtype"]
+            config.NORM_BETA = c["beta"]
+            edges = mcmc_gamma.postorder(mcmc_gamma.adjlist2nodes_dict(tree), root)[::-1]
+            rates = mcmc_gamma.get_siterates(0.8)
+            tm = [mcmc_gamma.get_prob_t(pi, tree, c["er"], r) for r in rates]
+            lnl, cache = ML_gamma.matML(pi, root, ll, edges, tm, P, N, 4)
+            path = mcmc_gamma.get_path2root(mcmc_gamma.adjlist2reverse_nodes_dict(tree), 3, root)
+            l2, _ = ML_gamma.cache_matML(pi, root, ll, cache, path, edges, tm, P, N, 4)
+        else:
+            edges = oracle.edge_order(tree, root, N)
+            rates = oracle.site_rates(0.8)
+            tm = [oracle.prob_t(c["model"], c["dtype"] == "bin", pi, tree, c["er"], r, beta=c["beta"]) for r in rates]
+            lnl, cache = oracle.mat_ml(pi, root, ll, edges, tm, P, N)
+            path = oracle.path_to_root(oracle.parent_of(tree), 3, root)
+            l2, _ = oracle.cache_mat_ml(pi, root, ll, cache, path, edges, tm, P, N)
+        rec.update(golden_io.random_vectors(i, c, edges, rates, tm, lnl, path, l2))
+    np.savez(out, **rec)
+
+
+if __name__ == "__main__" and len(sys.argv) > 1 and sys.argv[1] == "--random-inputs":
+    # python tests/golden/make_golden.py --random-inputs [OUT] [reference|oracle]
+    random_input_vectors(sys.argv[2] if len(sys.argv) > 2 else os.path.join(HERE, "random_inputs.npz"),
+                         sys.argv[3] if len(sys.argv) > 3 else "reference")

@@ -157,9 +157,7 @@ def test_unmodified_reference_driver_on_compat_modules(golden_cases, fake_backen
     `ML_gamma` from cybayes_b200/compat and produces its recorded per-generation output."""
     script = os.path.join(REPO, "oracle", "_ref", "mat_mcmc_gamma.code")
     if not os.path.exists(script):
-        script = "/root/reference/mat_mcmc_gamma.py"
-    if not os.path.exists(script):
-        pytest.skip("no reference driver available")
+        pytest.skip("no reference driver available (oracle/build_ref.sh)")
     monkeypatch.syspath_prepend(os.path.join(REPO, "cybayes_b200", "compat"))
     names = ("config", "utils", "mcmc_gamma", "ML_gamma", "mcmc", "ML")
     for m in names:

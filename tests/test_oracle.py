@@ -105,48 +105,37 @@ def test_gtr_eigen_route_matches_expm():
             np.testing.assert_allclose(b, a, rtol=5e-10, atol=1e-15)
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REPO, "oracle", "_ref")), reason="oracle/_ref not built")
-def test_oracle_against_compiled_reference_on_random_inputs():
-    """Fresh interpreter (the reference's top-level module names must not leak into this one):
-    random tree / data, the compiled reference's get_prob_t + matML + cache_matML vs the oracle."""
-    code = r'''
-import sys, random
-import numpy as np
-sys.path.insert(0, "oracle/_ref"); sys.path.insert(0, "oracle")
-import config, mcmc_gamma, ML_gamma
-import pruning_oracle as oracle
-rng = np.random.default_rng(5)
-for S, model, dtype in ((2, "F81", "bin"), (5, "F81", "multi"), (5, "JC", "multi"), (4, "GTR", "multi")):
-    n_taxa, n_sites = 11, 57
-    config.N_TAXA, config.N_CHARS, config.N_SITES, config.MODEL, config.IN_DTYPE = n_taxa, S, n_sites, model, dtype
-    nodes, nxt, tree = list(range(1, n_taxa + 1)), n_taxa + 1, {}
-    while len(nodes) > 1:
-        a = nodes.pop(int(rng.integers(len(nodes)))); b = nodes.pop(int(rng.integers(len(nodes))))
-        tree[nxt, a] = float(rng.exponential(0.1)); tree[nxt, b] = float(rng.exponential(0.1)); nodes.append(nxt); nxt += 1
-    root = nxt - 1
-    pi = rng.dirichlet(np.ones(S)) if model != "JC" else np.repeat(1.0 / S, S)
-    er = rng.dirichlet(np.ones(S * (S - 1) // 2))
-    config.NORM_BETA = 1 / (1 - np.dot(pi, pi))
-    eye = np.vstack([np.eye(S), np.ones(S)])
-    ll = {t: np.ascontiguousarray(eye[rng.integers(0, S + 1, n_sites)].T) for t in range(1, n_taxa + 1)}
-    edges = mcmc_gamma.postorder(mcmc_gamma.adjlist2nodes_dict(tree), root)[::-1]
-    assert edges == oracle.edge_order(tree, root, n_taxa)
-    rates = mcmc_gamma.get_siterates(0.8)
-    assert rates == oracle.site_rates(0.8)
-    tm_ref = [mcmc_gamma.get_prob_t(pi, tree, er, r) for r in rates]
-    tm = [oracle.prob_t(model, dtype == "bin", pi, tree, er, r, beta=config.NORM_BETA) for r in rates]
-    for k in range(4):
-        for e in tree:
-            assert np.array_equal(np.asarray(tm_ref[k][e]), tm[k][e]), (model, e)
-    l_ref, c_ref = ML_gamma.matML(pi, root, ll, edges, tm_ref, n_sites, n_taxa, 4)
-    l_or, c_or = oracle.mat_ml(pi, root, ll, edges, tm, n_sites, n_taxa)
-    assert l_ref == l_or, (l_ref, l_or)
-    path = mcmc_gamma.get_path2root(mcmc_gamma.adjlist2reverse_nodes_dict(tree), 3, root)
-    assert path == oracle.path_to_root(oracle.parent_of(tree), 3, root)
-    l2_ref, _ = ML_gamma.cache_matML(pi, root, ll, c_ref, path, edges, tm_ref, n_sites, n_taxa, 4)
-    l2_or, _ = oracle.cache_mat_ml(pi, root, ll, c_or, path, edges, tm, n_sites, n_taxa)
-    assert l2_ref == l2_or == l_ref
-print("OK")
-'''
-    res = subprocess.run([sys.executable, "-c", code], cwd=REPO, capture_output=True, text=True)
-    assert res.returncode == 0 and "OK" in res.stdout, res.stderr[-2000:]
+def _assert_same_vectors(got, want):
+    keys = sorted(k for k in want if k != "source")
+    assert sorted(k for k in got if k != "source") == keys
+    for k in keys:
+        assert got[k].dtype == want[k].dtype and np.array_equal(got[k], want[k]), k
+
+
+def test_oracle_against_compiled_reference_on_random_inputs(tmp_path):
+    """Seeded random trees and data (golden_io.random_inputs): the oracle's edge order, category rates, P(t) of every
+    edge, matML and cache_matML equal, bit for bit, the vectors stored in tests/golden/random_inputs.npz
+    (make_golden.py --random-inputs).  Its `source` entry says what computed them: "oracle" means the oracle itself,
+    recorded while it had none of its own changes since this test held it bit-equal to the compiled reference on these
+    inputs (DESIGN.md section 4), so the stored file pins that agreement.  Where the compiled reference is built
+    (oracle/_ref) it is run again, in a fresh interpreter so that its top-level module names do not leak into this
+    one, and must reproduce the stored vectors too."""
+    want = dict(np.load(golden_io.RANDOM_VECTORS))
+    got = {}
+    for i, c in enumerate(golden_io.random_inputs()):
+        tree, root, pi, ll, N, P = c["tree"], c["root"], c["pi"], c["ll"], c["n_taxa"], c["n_sites"]
+        edges = oracle.edge_order(tree, root, N)
+        rates = oracle.site_rates(0.8)
+        tm = [oracle.prob_t(c["model"], c["dtype"] == "bin", pi, tree, c["er"], r, beta=c["beta"]) for r in rates]
+        lnl, cache = oracle.mat_ml(pi, root, ll, edges, tm, P, N)
+        path = oracle.path_to_root(oracle.parent_of(tree), 3, root)
+        l2, _ = oracle.cache_mat_ml(pi, root, ll, cache, path, edges, tm, P, N)
+        assert l2 == lnl
+        got.update(golden_io.random_vectors(i, c, edges, rates, tm, lnl, path, l2))
+    _assert_same_vectors(got, want)
+    if os.path.exists(os.path.join(REPO, "oracle", "_ref")):
+        out = tmp_path / "reference.npz"
+        res = subprocess.run([sys.executable, os.path.join(REPO, "tests", "golden", "make_golden.py"), "--random-inputs",
+                              str(out), "reference"], cwd=REPO, capture_output=True, text=True)
+        assert res.returncode == 0, res.stderr[-2000:]
+        _assert_same_vectors(dict(np.load(out)), want)
