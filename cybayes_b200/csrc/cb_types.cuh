@@ -9,7 +9,9 @@ namespace cb {
 // tips.  Its partial has only 3 x 3 possible values per rate category (state code of either tip: 0, 1,
 // missing), so it is never computed per site, stored or read: the parent looks its contribution up.
 // SRC_STACK (tiled 2-state kernel only): the child was pushed into a shared-memory tile buffer by an earlier op of the walk.
-enum SrcKind : int32_t { SRC_TIP = 0, SRC_BUFFER = 1, SRC_CARRIED = 2, SRC_CHERRY = 3, SRC_STACK = 4 };
+// SRC_SMALL (tiled 2-state kernel only): the child is a (tip, cherry) subtree that the parent's op computes itself, so it
+// costs no op of its own and no stack slot.  Its descriptor is not in any range; in_buf names it (an index into ops).
+enum SrcKind : int32_t { SRC_TIP = 0, SRC_BUFFER = 1, SRC_CARRIED = 2, SRC_CHERRY = 3, SRC_STACK = 4, SRC_SMALL = 5 };
 
 constexpr int CB_S2_MAX_CATS = 4;            // rate categories of the 2-state kernels (1 or 4)
 constexpr int32_t CB_LIB_SLOT = 1 << 30;     // P-slot ids with this bit address the library's own pool
@@ -31,7 +33,7 @@ struct OpDesc {
   int32_t crec_out[2];                     // library record that must keep a copy of those P, or -1
   // tiled 2-state kernel (kernels_s2t.cuh)
   int32_t out_buf;                         // shared-memory tile buffer receiving the result, or -1
-  int32_t in_buf[2];                       // kind == SRC_STACK: tile buffer holding the child
+  int32_t in_buf[2];                       // kind == SRC_STACK: tile buffer holding the child; SRC_SMALL: its op index
   int32_t spill;                           // bit 0: stored AND read back inside the same launch (plain stores);
                                            // bit 1: out_buf is a stack slot (the result is popped by a later op)
   int32_t frec_out;                        // library record that must keep a copy of THIS op's two edges' P, or -1

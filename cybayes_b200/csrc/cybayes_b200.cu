@@ -162,6 +162,7 @@ struct EvalPlan {
   std::vector<PlanLaunch> launches;
   int64_t bytes_written = 0, bytes_read = 0;
   int n_stored = 0, n_buffer_reads = 0, n_stack = 0, n_spills = 0, n_cherries = 0, n_small_recs = 0;
+  int n_inlined = 0;   // ops computed inside their parent's op (SRC_SMALL): in `ops` for their descriptor, in no range
   uint64_t stamp = 0;
 };
 constexpr int PLAN_FLAG_MASK = CB_EVAL_WANT_SNAPSHOT | CB_EVAL_STORE_ROOT | CB_EVAL_FORCE_LEVELS | CB_EVAL_FORCE_WALK | CB_EVAL_NO_FOLD;
@@ -1078,7 +1079,13 @@ static int build_plan(cb_ctx* c, const Snapshot* sin, int n_lists, const int32_t
   plan.ops.clear(); plan.ranges.clear(); plan.launches.clear();
   plan.bytes_written = plan.bytes_read = 0;
   plan.n_stored = plan.n_buffer_reads = plan.n_stack = plan.n_spills = plan.n_cherries = plan.n_small_recs = 0;
+  plan.n_inlined = 0;
   const int64_t tip_row_bytes = c->P * c->code_bytes;
+  // small subtrees (children: tips / cherries) of a cache-kept pass are kept as records instead of being stored
+  const bool small_recs = c->s2_tiled && c->s2t_small_recs && want_snap;
+  auto snap_cherry = [&](int nd) {   // the input snapshot holds node nd as a record (a folded cherry or a small subtree)
+    return fold && sin && nd < (int)sin->cherry_of_node.size() && sin->cherry_of_node[nd] >= 0;
+  };
 
   struct LOp { int32_t node, caller; int32_t child[2], folded[2]; };
   std::vector<LOp> L;
@@ -1088,6 +1095,8 @@ static int build_plan(cb_ctx* c, const Snapshot* sin, int n_lists, const int32_t
   std::vector<int> seg_of;     // op -> segment (0 = top / whole list, s + 1 = cut subtree s)
   std::vector<int> f;          // DP table [op][k]
   std::vector<char> read_back;
+  std::vector<int> small_of;   // op -> its child (0 / 1) that it computes itself (SRC_SMALL), or -1
+  std::vector<char> inlined;   // op -> computed inside its parent's op
   bool single_launch = true;
 
   for (int li = 0; li < n_lists; ++li) {
@@ -1184,6 +1193,33 @@ static int build_plan(cb_ctx* c, const Snapshot* sin, int n_lists, const int32_t
       if (n_lists > 1 && sched == SCHED_LEVELS) return fail("cb_eval_batch: candidate %d is not a chain (level schedule forced)", li);
     }
 
+    // Tiled kernel: a (tip, cherry) subtree that is not stored is computed inside its parent's op (SRC_SMALL) when the
+    // parent runs in the same range and its other child is a tip or the op carried into it -- the same arithmetic
+    // without an op of its own (image, dispatch, rescale, loop iteration) and without a stack slot.
+    small_of.assign(n, -1);
+    inlined.assign(n, 0);
+    int n_inl = 0;
+    auto is_cherry = [&](int j, int kx) {   // the child resolves to SRC_CHERRY (below)
+      const int ch = L[j].child[kx];
+      return ch > N && (L[j].folded[kx] >= 0 || (kid[kx][j] < 0 && snap_cherry(ch)));
+    };
+    auto pick_small = [&] {
+      if (!c->s2_tiled) return;
+      for (int j = 0; j < n; ++j)
+        for (int kx = 1; kx >= 0 && small_of[j] < 0; --kx) {
+          const int s = kid[kx][j], o = kid[1 - kx][j];
+          if (s < 0 || seg_of[s] != seg_of[j]) continue;
+          const bool tip_cherry = (L[s].child[0] <= N && is_cherry(s, 1)) || (L[s].child[1] <= N && is_cherry(s, 0));
+          // not stored: likelihood-only pass, a recomputed record, or kept as a record (make_rec below; checked there)
+          const bool unstored = !want_snap || L[s].caller < 0 || small_recs;
+          const bool sibling_ok = L[j].child[1 - kx] <= N || (o >= 0 && seg_of[o] == seg_of[j]);
+          if (tip_cherry && unstored && sibling_ok) {
+            small_of[j] = kx;
+            inlined[s] = 1;
+            n_inl++;
+          }
+        }
+    };
     order.resize(n);
     for (int j = 0; j < n; ++j) order[j] = j;
     seg_of.assign(n, 0);
@@ -1247,14 +1283,19 @@ static int build_plan(cb_ctx* c, const Snapshot* sin, int n_lists, const int32_t
             }
           }
         }
+        pick_small();
+        // children the walk visits: a cut root lives in another launch and is read from its buffer; an inlined subtree
+        // is computed by its parent, like a tip
+        auto walk_kid = [&](int kx, int j) {
+          const int a = kid[kx][j];
+          return a >= 0 && seg_of[a] == seg_of[j] && !inlined[a] ? a : -1;
+        };
         // visiting order per segment: f[j][k] = fewest read-backs in j's subtree (inside its segment) with k free stack
         // slots; of two internal children the first visited is pushed (or read back when k == 0), the second carried
         f.assign((size_t)n * (K + 1), 0);
         first_kid.assign((size_t)n * (K + 1), 0);
         for (int j = 0; j < n; ++j) {
-          int a = kid[0][j], b2 = kid[1][j];
-          if (a >= 0 && seg_of[a] != seg_of[j]) a = -1;    // a cut root: lives in another launch, read from its buffer
-          if (b2 >= 0 && seg_of[b2] != seg_of[j]) b2 = -1;
+          const int a = walk_kid(0, j), b2 = walk_kid(1, j);
           for (int kk = 0; kk <= K; ++kk) {
             int& fj = f[(size_t)j * (K + 1) + kk];
             if (a >= 0 && b2 >= 0) {
@@ -1287,9 +1328,7 @@ static int build_plan(cb_ctx* c, const Snapshot* sin, int n_lists, const int32_t
           while (!fr.empty()) {
             Frame& t = fr.back();
             const int j = t.j, kk = t.k;
-            int a = kid[0][j], b2 = kid[1][j];
-            if (a >= 0 && seg_of[a] != seg_of[j]) a = -1;
-            if (b2 >= 0 && seg_of[b2] != seg_of[j]) b2 = -1;
+            const int a = walk_kid(0, j), b2 = walk_kid(1, j);
             if (a >= 0 && b2 >= 0) {
               const int fk = first_kid[(size_t)j * (K + 1) + kk];
               const bool push = kk > 0 && !(fk & 2);
@@ -1318,10 +1357,19 @@ static int build_plan(cb_ctx* c, const Snapshot* sin, int n_lists, const int32_t
           }
           emit(n - 1);
         }
-        REQUIRE((int)out.size() == n, "internal error: walk order covers %d of %d ops", (int)out.size(), n);
+        REQUIRE((int)out.size() == n - n_inl, "internal error: walk order covers %d of %d ops", (int)out.size(), n - n_inl);
+        for (int j = 0; j < n; ++j)
+          if (inlined[j]) out.push_back(j);   // descriptors only: after the ops the ranges run
         order = out;
       }
+    } else if (sched == SCHED_CHAIN) {
+      pick_small();   // only the first op of a chain can be such a subtree; its parent takes it beside a tip
+      if (n_inl > 0) {
+        std::stable_partition(order.begin(), order.end(), [&](int j) { return !inlined[j]; });
+      }
     }
+    const int n_exec = n - n_inl;   // positions [n_exec, n): inlined ops
+    plan.n_inlined += n_inl;
     pos_of.assign(n, 0);
     for (int p = 0; p < n; ++p) pos_of[order[p]] = p;
     range_id.assign(n, 0);   // by position
@@ -1340,7 +1388,7 @@ static int build_plan(cb_ctx* c, const Snapshot* sin, int n_lists, const int32_t
       PlanOp& po = plan.ops[base + p];
       po.node = L[j].node;
       po.is_root = (j == n - 1);
-      REQUIRE(!po.is_root || p == n - 1, "internal error: root is not last");
+      REQUIRE(!po.is_root || p == n_exec - 1, "internal error: root is not last");
       po.keep = po.stream = po.spill = po.pushed = po.make_rec = 0;
       po.synthetic = L[j].caller < 0 ? 1 : 0;
       po.out_buf = po.pf_buf = -1;
@@ -1356,6 +1404,9 @@ static int build_plan(cb_ctx* c, const Snapshot* sin, int n_lists, const int32_t
           pc.kind = SRC_CHERRY;
           pc.ref = L[j].folded[kx];
           plan.bytes_read += 2 * tip_row_bytes;
+        } else if (small_of[j] == kx) {
+          pc.kind = SRC_SMALL;
+          pc.ref = base + pos_of[kid[kx][j]];   // its descriptor
         } else if (kid[kx][j] >= 0) {
           const int jj = kid[kx][j], pp = pos_of[jj];
           if (same_range(pp, p) && pp == p - 1) {
@@ -1374,7 +1425,7 @@ static int build_plan(cb_ctx* c, const Snapshot* sin, int n_lists, const int32_t
             plan.n_buffer_reads++;
           }
         } else {
-          const bool rec = fold && sin && ch < (int)sin->cherry_of_node.size() && sin->cherry_of_node[ch] >= 0;
+          const bool rec = snap_cherry(ch);
           pc.kind = rec ? SRC_CHERRY : SRC_BUFFER;
           pc.ref = ~ch;
           plan.bytes_read += rec ? 2 * tip_row_bytes : (int64_t)c->buffer_bytes;
@@ -1402,7 +1453,7 @@ static int build_plan(cb_ctx* c, const Snapshot* sin, int n_lists, const int32_t
         if (po.spill) plan.n_spills++;
       }
       // small subtrees (children: tips / cherries) are not stored: the returned snapshot keeps a record
-      if (c->s2_tiled && c->s2t_small_recs && want_snap && po.keep && !po.is_root && !po.synthetic && read_back[j] == 0 &&
+      if (small_recs && po.keep && !po.is_root && !po.synthetic && read_back[j] == 0 &&
           (po.ch[0].kind == SRC_TIP || po.ch[0].kind == SRC_CHERRY) && po.ch[1].kind == SRC_CHERRY) {
         po.keep = 0;
         po.stream = 0;
@@ -1411,6 +1462,8 @@ static int build_plan(cb_ctx* c, const Snapshot* sin, int n_lists, const int32_t
         plan.n_stored--;
         plan.n_small_recs++;
       }
+      // an inlined op has no store of its own: a buffer given to it would enter the snapshot unwritten
+      REQUIRE(!inlined[j] || !po.keep, "internal error: inlined node %d would be stored", po.node);
       if (c->s2_tiled) {
         if (push_slot[j] >= 0 && !po.is_root) { po.out_buf = push_slot[j]; po.pushed = 1; }
         else if (c->s2t_bulk && po.keep && !po.spill) { po.out_buf = staging_rr; staging_rr ^= 1; }
@@ -1459,10 +1512,10 @@ static int build_plan(cb_ctx* c, const Snapshot* sin, int n_lists, const int32_t
       }
       plan.launches.push_back({start, (int)plan.ranges.size(), mx, nb});
       const int tb = segs.back().second;
-      plan.ranges.push_back(RangeDesc{base + tb, base + n, li, 0});
-      plan.launches.push_back({(int)plan.ranges.size() - 1, (int)plan.ranges.size(), n - tb, bufs_of(tb, n)});
+      plan.ranges.push_back(RangeDesc{base + tb, base + n_exec, li, 0});
+      plan.launches.push_back({(int)plan.ranges.size() - 1, (int)plan.ranges.size(), n_exec - tb, bufs_of(tb, n_exec)});
     } else if (sched != SCHED_LEVELS) {
-      plan.ranges.push_back(RangeDesc{base, base + n, li, 0});
+      plan.ranges.push_back(RangeDesc{base, base + n_exec, li, 0});
     } else {
       single_launch = false;
       level_of.assign(n, 1);
@@ -1642,6 +1695,9 @@ static int eval_impl(cb_ctx* c, int snapshot_in, int n_lists, const int32_t* off
             op.src_scale[kx] = bf.scale;
           }
           break;
+        case SRC_SMALL:
+          op.in_buf[kx] = pc.ref;
+          break;
         case SRC_STACK:
           if (po.pf_buf >= 0 && kx == 1) {   // a prefetched stored partial: the source is a buffer, the op reads the tile buffer
             op.in_buf[kx] = po.pf_buf;
@@ -1763,7 +1819,7 @@ static int eval_impl(cb_ctx* c, int snapshot_in, int n_lists, const int32_t* off
   c->timing_valid = c->timing;
   c->last_bytes_written = plan->bytes_written;
   c->last_bytes_read = plan->bytes_read;
-  c->last_counts[0] = total_ops; c->last_counts[1] = plan->n_stored; c->last_counts[2] = plan->n_buffer_reads;
+  c->last_counts[0] = total_ops - plan->n_inlined; c->last_counts[1] = plan->n_stored; c->last_counts[2] = plan->n_buffer_reads;
   c->last_counts[3] = plan->n_stack; c->last_counts[4] = plan->n_spills; c->last_counts[5] = plan->n_cherries;
   c->last_counts[6] = (int)plan->launches.size(); c->last_counts[7] = plan->n_small_recs;
 

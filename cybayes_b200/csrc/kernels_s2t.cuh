@@ -46,7 +46,8 @@ struct S2TImage {
   char* dst;                 // tile-layout partial buffer, or nullptr (not stored)
   const char* src[2];        // SRC_BUFFER: tile-layout partial buffer; SRC_TIP: code row
   const void* rows[4];       // code rows the op reads, at fixed positions: child 0 -> [0] (tip / cherry tip a), [1] (cherry
-                             // tip b); child 1 -> [2], [3]; unused positions point at a valid row (loaded, ignored)
+                             // tip b); child 1 -> [2], [3] (SRC_SMALL: see s2t_rank); unused positions point at a valid
+                             // row (loaded, ignored)
   int32_t kind[2];           // canonical order (s2t_rank): the host swaps the children when needed
   int32_t is_root;
   int32_t combo;             // S2TCombo: the pair of child kinds, selects the specialised op body
@@ -58,19 +59,29 @@ struct S2TImage {
 };
 static_assert(sizeof(S2TImage) == 1408, "S2TImage must stay 1408 bytes (a multiple of 16)");
 
-// Children of an op are kept in a canonical order (products and exponent sums commute exactly), which leaves ten
+// Children of an op are kept in a canonical order (products and exponent sums commute exactly), which leaves twelve
 // possible pairs of child kinds; each has its own straight-line op body in the kernel.
+//
+// An inlined (tip, cherry) subtree (SRC_SMALL) is always child 1, beside a carried child or a tip.  Its op image holds
+// three children's worth of tables: tab[0] = child 0's P rows (4C doubles), the parent's P rows for the subtree (4C),
+// the subtree's P rows for its tip (4C); tab[1] = the subtree's cherry table.  Code rows: [0] child 0's tip, [1] the
+// subtree's tip, [2] and [3] the tips of its cherry.
 __host__ __device__ constexpr int s2t_rank(int kind) {
-  return kind == SRC_CARRIED ? 0 : kind == SRC_STACK ? 1 : kind == SRC_BUFFER ? 2 : kind == SRC_TIP ? 3 : 4;
+  return kind == SRC_CARRIED ? 0 : kind == SRC_STACK ? 1 : kind == SRC_BUFFER ? 2 : kind == SRC_TIP ? 3 : kind == SRC_CHERRY ? 4 : 5;
 }
 enum S2TCombo : int32_t {
   S2T_CARRIED_STACK = 0, S2T_CARRIED_BUFFER, S2T_CARRIED_TIP, S2T_CARRIED_CHERRY, S2T_BUFFER_BUFFER, S2T_BUFFER_TIP,
-  S2T_BUFFER_CHERRY, S2T_TIP_TIP, S2T_TIP_CHERRY, S2T_CHERRY_CHERRY, S2T_N_COMBOS
+  S2T_BUFFER_CHERRY, S2T_TIP_TIP, S2T_TIP_CHERRY, S2T_CHERRY_CHERRY, S2T_CARRIED_SMALL, S2T_TIP_SMALL, S2T_N_COMBOS
 };
+// does an op whose children have kinds k0, k1 (canonical order) read code row q of its image?
+__host__ __device__ inline bool s2t_row_used(int k0, int k1, int q) {
+  return q == 0 ? (k0 == SRC_TIP || k0 == SRC_CHERRY) : q == 1 ? (k0 == SRC_CHERRY || k1 == SRC_SMALL)
+                                                               : (k1 == SRC_CHERRY || k1 == SRC_SMALL || (q == 2 && k1 == SRC_TIP));
+}
 __host__ __device__ inline int s2t_combo(int k0, int k1) {   // kinds in canonical order; -1: not a pair the walk produces
-  if (k0 == SRC_CARRIED) return k1 == SRC_STACK ? S2T_CARRIED_STACK : k1 == SRC_BUFFER ? S2T_CARRIED_BUFFER : k1 == SRC_TIP ? S2T_CARRIED_TIP : k1 == SRC_CHERRY ? S2T_CARRIED_CHERRY : -1;
+  if (k0 == SRC_CARRIED) return k1 == SRC_STACK ? S2T_CARRIED_STACK : k1 == SRC_BUFFER ? S2T_CARRIED_BUFFER : k1 == SRC_TIP ? S2T_CARRIED_TIP : k1 == SRC_CHERRY ? S2T_CARRIED_CHERRY : k1 == SRC_SMALL ? S2T_CARRIED_SMALL : -1;
   if (k0 == SRC_BUFFER) return k1 == SRC_BUFFER ? S2T_BUFFER_BUFFER : k1 == SRC_TIP ? S2T_BUFFER_TIP : k1 == SRC_CHERRY ? S2T_BUFFER_CHERRY : -1;
-  if (k0 == SRC_TIP) return k1 == SRC_TIP ? S2T_TIP_TIP : k1 == SRC_CHERRY ? S2T_TIP_CHERRY : -1;
+  if (k0 == SRC_TIP) return k1 == SRC_TIP ? S2T_TIP_TIP : k1 == SRC_CHERRY ? S2T_TIP_CHERRY : k1 == SRC_SMALL ? S2T_TIP_SMALL : -1;
   if (k0 == SRC_CHERRY) return k1 == SRC_CHERRY ? S2T_CHERRY_CHERRY : -1;
   return -1;
 }
@@ -165,6 +176,12 @@ __global__ void __launch_bounds__(32) s2t_image_kernel(const LaunchConst k, int 
       im->rows[2 * ch] = kind == SRC_TIP ? op->src[ch] : kind == SRC_CHERRY ? op->ctip[ch][0] : k.codes;
       im->rows[2 * ch + 1] = kind == SRC_CHERRY ? op->ctip[ch][1] : k.codes;
     }
+    if (op->kind[1] == SRC_SMALL) {   // the subtree's own descriptor holds its children in canonical order: (tip, cherry)
+      const OpDesc* sub = k.ops + op->in_buf[1];
+      im->rows[1] = sub->src[0];
+      im->rows[2] = sub->ctip[1][0];
+      im->rows[3] = sub->ctip[1][1];
+    }
     im->kind[0] = op->kind[0]; im->kind[1] = op->kind[1];
     im->is_root = op->is_root;
     im->combo = s2t_combo(op->kind[0], op->kind[1]);
@@ -188,26 +205,31 @@ __global__ void __launch_bounds__(32) s2t_image_kernel(const LaunchConst k, int 
       const int e = idx & 3, c = (idx >> 2) % C, ch = idx / (4 * C);
       k.pmats_lib[((int64_t)op->frec_out * 2 * C + ch * C + c) * 4 + e] = __ldg(s2_pmat(k, op->pslot[ch][c]) + e);
     }
-  // P matrices of internal and tip children (one thread per child, category and row)
-  for (int idx = t; idx < 4 * C; idx += 32) {
-    const int i = idx & 1, c = (idx >> 1) % C, ch = idx / (2 * C);
+  // P matrices of internal and tip children (one thread per child, category and row); an inlined subtree's rows go
+  // to tab[0] behind child 0's, followed by the rows of the subtree's edge to its tip
+  for (int idx = t; idx < 6 * C; idx += 32) {
+    const int i = idx & 1, c = (idx >> 1) % C, ch = min(idx / (2 * C), 1);
     const int kind = op->kind[ch];
-    if (kind == SRC_CHERRY) continue;
-    const double2 pr = __ldg(reinterpret_cast<const double2*>(s2_pmat(k, op->pslot[ch][c])) + i);
-    reinterpret_cast<double2*>(&im->tab[ch][0])[c * 2 + i] = pr;   // tips use the same rows (see s2t_child)
-    (void)kind;
+    if (kind == SRC_CHERRY || (idx >= 4 * C && kind != SRC_SMALL)) continue;
+    const int32_t slot = idx >= 4 * C ? k.ops[op->in_buf[1]].pslot[0][c] : op->pslot[ch][c];
+    const double2 pr = __ldg(reinterpret_cast<const double2*>(s2_pmat(k, slot)) + i);
+    if (kind == SRC_SMALL) reinterpret_cast<double2*>(&im->tab[0][0])[(idx >= 4 * C ? 4 * C : 2 * C) + c * 2 + i] = pr;
+    else reinterpret_cast<double2*>(&im->tab[ch][0])[c * 2 + i] = pr;   // tips use the same rows (see s2t_child)
   }
-  // lookup tables of folded cherries (one thread per child and pair of tip codes)
+  // lookup tables of folded cherries (one thread per child and pair of tip codes); an inlined subtree's cherry is
+  // child 1 of the subtree's descriptor
   for (int idx = t; idx < 18; idx += 32) {
     const int q = idx % 9, ch = idx / 9;
-    if (op->kind[ch] != SRC_CHERRY) continue;
+    if (op->kind[ch] != SRC_CHERRY && op->kind[ch] != SRC_SMALL) continue;
+    const OpDesc* cd = op->kind[ch] == SRC_SMALL ? k.ops + op->in_buf[ch] : op;
+    const int cc = op->kind[ch] == SRC_SMALL ? 1 : ch;
     const int ca = q / 3, cb_ = q - 3 * ca;
     double L[C][2];
     int mh = 0;
 #pragma unroll
     for (int c = 0; c < C; ++c) {
-      const double2* pa = reinterpret_cast<const double2*>(s2_pmat(k, op->cslot[ch][0][c]));
-      const double2* pb = reinterpret_cast<const double2*>(s2_pmat(k, op->cslot[ch][1][c]));
+      const double2* pa = reinterpret_cast<const double2*>(s2_pmat(k, cd->cslot[cc][0][c]));
+      const double2* pb = reinterpret_cast<const double2*>(s2_pmat(k, cd->cslot[cc][1][c]));
 #pragma unroll
       for (int j = 0; j < 2; ++j) {
         L[c][j] = s2_tip_term(__ldg(pa + j), ca) * s2_tip_term(__ldg(pb + j), cb_);
@@ -221,7 +243,7 @@ __global__ void __launch_bounds__(32) s2t_image_kernel(const LaunchConst k, int 
 #pragma unroll
     for (int c = 0; c < C; ++c) {
       const double l0 = L[c][0] * f, l1 = L[c][1] * f;
-      const double2* pp = reinterpret_cast<const double2*>(s2_pmat(k, op->pslot[ch][c]));
+      const double2* pp = reinterpret_cast<const double2*>(s2_pmat(k, cd->pslot[cc][c]));
 #pragma unroll
       for (int i = 0; i < 2; ++i) {
         const double2 pr = __ldg(pp + i);
@@ -229,8 +251,9 @@ __global__ void __launch_bounds__(32) s2t_image_kernel(const LaunchConst k, int 
       }
     }
     tab[2 * C] = (double)x;
-    // a cherry that stays in the returned cache keeps its own copy of its two edges' P matrices
-    if (q == 0 && op->crec_out[ch] >= 0) {
+    // a cherry that stays in the returned cache keeps its own copy of its two edges' P matrices (an inlined subtree's
+    // descriptor gets an image of its own, which writes its records' copies)
+    if (q == 0 && cd == op && op->crec_out[ch] >= 0) {
       double* out = k.pmats_lib + (int64_t)op->crec_out[ch] * 2 * C * 4;
 #pragma unroll
       for (int tt = 0; tt < 2; ++tt)
@@ -327,6 +350,54 @@ __device__ __forceinline__ void s2t_child(const S2TImage& im, const double (&cur
     }
 #pragma unroll
     for (int v = 0; v < V; ++v) if (FIRST) e_in[v] = 0;
+  } else if constexpr (KIND == SRC_SMALL) {
+    // A (tip, cherry) subtree, computed exactly as its own TIP_CHERRY op would (tip rows, times the cherry's row, then
+    // the same power-of-two rescale) and then fed through the parent's P rows like a carried child.
+    static_assert(CH == 1 && !FIRST, "an inlined subtree is child 1");
+    const double2* pt = reinterpret_cast<const double2*>(&im.tab[0][0]) + 4 * C;   // subtree -> its tip
+    const double2* pm = reinterpret_cast<const double2*>(&im.tab[0][0]) + 2 * C;   // parent -> subtree
+    double L[V][C][2];
+    int se[V];
+#pragma unroll
+    for (int v = 0; v < V; ++v) {
+      const unsigned cd = codes[1 * (S2T_W * V) + v * S2T_W + lane];
+      const double m0 = cd == 1u ? 0.0 : 1.0, m1 = cd == 0u ? 0.0 : 1.0;
+#pragma unroll
+      for (int c = 0; c < C; ++c)
+#pragma unroll
+        for (int i = 0; i < 2; ++i) {
+          const double2 pr = pt[c * 2 + i];
+          L[v][c][i] = fma(pr.y, m1, pr.x * m0);
+        }
+      const unsigned ca = min((unsigned)codes[2 * (S2T_W * V) + v * S2T_W + lane], 2u);
+      const unsigned cb_ = min((unsigned)codes[3 * (S2T_W * V) + v * S2T_W + lane], 2u);
+      const double* tab = pbase + (ca * 3 + cb_) * (2 * C + 1);
+      int mh = 0;
+#pragma unroll
+      for (int c = 0; c < C; ++c)
+#pragma unroll
+        for (int i = 0; i < 2; ++i) {
+          L[v][c][i] *= tab[c * 2 + i];
+          mh = c == 0 && i == 0 ? __double2hiint(L[v][0][0]) : max(mh, __double2hiint(L[v][c][i]));
+        }
+      const int be = (mh >> 20) & 0x7ff;
+      const int x = (be == 0 || be == 0x7ff) ? 0 : be - 1023;
+      const double f = pow2_neg(x);
+#pragma unroll
+      for (int c = 0; c < C; ++c) { L[v][c][0] *= f; L[v][c][1] *= f; }
+      se[v] = (int)tab[2 * C] + x;
+    }
+#pragma unroll
+    for (int c = 0; c < C; ++c) {
+#pragma unroll
+      for (int i = 0; i < 2; ++i) {
+        const double2 pr = pm[c * 2 + i];
+#pragma unroll
+        for (int v = 0; v < V; ++v) acc[v][c][i] *= fma(pr.y, L[v][c][1], pr.x * L[v][c][0]);
+      }
+    }
+#pragma unroll
+    for (int v = 0; v < V; ++v) e_in[v] += se[v];
   } else {  // folded cherry: the pair of tip codes selects a precomputed row
 #pragma unroll
     for (int v = 0; v < V; ++v) {
@@ -477,6 +548,8 @@ __global__ void __launch_bounds__(S2T_THREADS / V, MINB) prune_s2t_kernel(const 
         CB_S2T_CASE(S2T_BUFFER_CHERRY, SRC_BUFFER, SRC_CHERRY)
         CB_S2T_CASE(S2T_TIP_TIP, SRC_TIP, SRC_TIP)
         CB_S2T_CASE(S2T_TIP_CHERRY, SRC_TIP, SRC_CHERRY)
+        CB_S2T_CASE(S2T_CARRIED_SMALL, SRC_CARRIED, SRC_SMALL)
+        CB_S2T_CASE(S2T_TIP_SMALL, SRC_TIP, SRC_SMALL)
         default:
           s2t_pair<C, V, SRC_CHERRY, SRC_CHERRY>(im, cur, cur_e, codes, mybufs, tile_off, lane, out, e_in);
           break;
@@ -577,11 +650,10 @@ __global__ void __launch_bounds__(S2T_THREADS / V, MINB) prune_s2t_kernel(const 
           const int c1 = (o + 2) / S2T_RING_OPS;
           const int e = (c1 + 2) * S2T_RING_OPS + (lane >> 2);
           if (lane < 4 * S2T_RING_OPS && e < nops && warp == c1 % n_active) {  // one warp per block and chunk does it
-            const OpDesc* __restrict__ dn = k.ops + rg.begin + e;
-            const int ch = (lane >> 1) & 1, t = lane & 1;
-            const int kind = dn->kind[ch];
-            const void* row = kind == SRC_TIP ? (t == 0 ? dn->src[ch] : nullptr) : (kind == SRC_CHERRY ? dn->ctip[ch][t] : nullptr);
-            if (row != nullptr) {
+            const S2TImage& ie = gimg[e];   // (the image kernel ran before this launch)
+            const int q = lane & 3;
+            if (s2t_row_used(ie.kind[0], ie.kind[1], q)) {
+              const void* row = ie.rows[q];
               const char* a = static_cast<const char*>(row) + (int64_t)blockIdx.x * S2T_WARPS * S2T_W;   // the block's 256 sites
               asm volatile("prefetch.global.L2 [%0];" ::"l"(a));
               asm volatile("prefetch.global.L2 [%0];" ::"l"(a + 128));
