@@ -1,7 +1,14 @@
-// Device-visible descriptors shared by the host scheduler and the pruning kernels.
+// Device-visible descriptors shared by the host scheduler and the pruning kernels.  Also compiled by the host compiler
+// alone (plan.cpp), so nothing here needs CUDA headers.
 #pragma once
 #include <stdint.h>
 #include "../../include/cybayes_b200.h"
+
+#ifdef __CUDACC__
+#define CB_HD __host__ __device__
+#else
+#define CB_HD
+#endif
 
 namespace cb {
 
@@ -76,6 +83,34 @@ struct LaunchConst {
   struct Mail* const* peer_mailbox;    // device array: every rank's mailbox (peer pointers opened through CUDA IPC)
   int32_t* comm_error;                 // set when a peer never delivered (timeout)
 };
+
+// ---- tiled 2-state kernel (kernels_s2t.cuh): tile geometry and the child kinds its op bodies take
+constexpr int S2T_W = 32;          // sites per tile
+constexpr int S2T_WARPS = 8;       // tiles per block (a warp owns V consecutive tiles: 8 / V warps per block)
+constexpr int S2T_THREADS = S2T_W * S2T_WARPS;
+constexpr int S2T_STAGING = 2;     // bulk-store path only: tile buffers 0..1 per warp rotate as store staging, stack slots follow
+
+// Children of an op are kept in a canonical order (products and exponent sums commute exactly), which leaves twelve
+// possible pairs of child kinds; each has its own straight-line op body in the kernel.
+//
+// An inlined (tip, cherry) subtree (SRC_SMALL) is always child 1, beside a carried child or a tip.  Its op image holds
+// three children's worth of tables: tab[0] = child 0's P rows (4C doubles), the parent's P rows for the subtree (4C),
+// the subtree's P rows for its tip (4C); tab[1] = the subtree's cherry table.  Code rows: [0] child 0's tip, [1] the
+// subtree's tip, [2] and [3] the tips of its cherry.
+CB_HD constexpr int s2t_rank(int kind) {
+  return kind == SRC_CARRIED ? 0 : kind == SRC_STACK ? 1 : kind == SRC_BUFFER ? 2 : kind == SRC_TIP ? 3 : kind == SRC_CHERRY ? 4 : 5;
+}
+enum S2TCombo : int32_t {
+  S2T_CARRIED_STACK = 0, S2T_CARRIED_BUFFER, S2T_CARRIED_TIP, S2T_CARRIED_CHERRY, S2T_BUFFER_BUFFER, S2T_BUFFER_TIP,
+  S2T_BUFFER_CHERRY, S2T_TIP_TIP, S2T_TIP_CHERRY, S2T_CHERRY_CHERRY, S2T_CARRIED_SMALL, S2T_TIP_SMALL, S2T_N_COMBOS
+};
+CB_HD inline int s2t_combo(int k0, int k1) {   // kinds in canonical order; -1: not a pair the walk produces
+  if (k0 == SRC_CARRIED) return k1 == SRC_STACK ? S2T_CARRIED_STACK : k1 == SRC_BUFFER ? S2T_CARRIED_BUFFER : k1 == SRC_TIP ? S2T_CARRIED_TIP : k1 == SRC_CHERRY ? S2T_CARRIED_CHERRY : k1 == SRC_SMALL ? S2T_CARRIED_SMALL : -1;
+  if (k0 == SRC_BUFFER) return k1 == SRC_BUFFER ? S2T_BUFFER_BUFFER : k1 == SRC_TIP ? S2T_BUFFER_TIP : k1 == SRC_CHERRY ? S2T_BUFFER_CHERRY : -1;
+  if (k0 == SRC_TIP) return k1 == SRC_TIP ? S2T_TIP_TIP : k1 == SRC_CHERRY ? S2T_TIP_CHERRY : k1 == SRC_SMALL ? S2T_TIP_SMALL : -1;
+  if (k0 == SRC_CHERRY) return k1 == SRC_CHERRY ? S2T_CHERRY_CHERRY : -1;
+  return -1;
+}
 
 constexpr int CB_MB_OUTS = 64;          // results per evaluation the fused all-reduce handles (larger batches use NCCL)
 struct Mail {

@@ -23,6 +23,7 @@
 #include <vector>
 
 #include "cb_types.cuh"
+#include "plan.h"
 #include "kernels_dmma.cuh"
 #include "kernels_dmma_rc.cuh"
 #include "kernels_general.cuh"
@@ -34,7 +35,7 @@ using namespace cb;
 
 // ------------------------------------------------------------------------------ errors
 static thread_local std::string g_err;
-static int fail(const char* fmt, ...) {
+int cb::fail(const char* fmt, ...) {
   char buf[1024];
   va_list ap;
   va_start(ap, fmt);
@@ -47,10 +48,6 @@ static int fail(const char* fmt, ...) {
   do {                                                                                        \
     cudaError_t e_ = (call);                                                                  \
     if (e_ != cudaSuccess) return fail("%s:%d %s: %s", __FILE__, __LINE__, #call, cudaGetErrorString(e_)); \
-  } while (0)
-#define REQUIRE(cond, ...)            \
-  do {                                \
-    if (!(cond)) return fail(__VA_ARGS__); \
   } while (0)
 
 
@@ -117,57 +114,6 @@ struct Buffer {
   int32_t* scale = nullptr;
   int refs = 0;
 };
-struct Snapshot {
-  std::vector<int32_t> buf_of_node;     // index by node id; -1 = absent
-  std::vector<int32_t> cherry_of_node;  // 2-state family: record of a folded cherry (never materialised), or -1
-  int refs = 0;
-};
-// A small subtree kept by a snapshot as a RECORD instead of a stored partial: its two children and, in the library's own
-// P pool at slots [rec * 2C, (rec + 1) * 2C), copies of the P matrices of its two child edges (child 0: C slots, child 1:
-// C slots).  A cherry (both children tips) is folded into its parent's lookup table; a node whose children are tips or
-// cherries (3 or 4 tips below it; tiled kernel only) is recomputed on the fly when a later dirty path needs it as a
-// sibling -- two table look-ups and a product per site instead of 68 bytes of HBM per site.  child[k] <= n_taxa: a tip;
-// otherwise the node id of a cherry that the same snapshot holds as a record.
-struct CherryRec {
-  int32_t tip[2] = {0, 0};   // (children; named tip for the common case)
-  int refs = 0;
-};
-
-// ---- evaluation plans (see build_plan)
-struct PlanChild {
-  int32_t kind;  // SrcKind
-  int32_t ref;   // SRC_TIP: tip id.  SRC_BUFFER: position of the producing op, or ~node (< 0) when the input snapshot
-                 // holds it.  SRC_CHERRY: caller's op index of the folded cherry, or ~node for a record of the input
-                 // snapshot.  SRC_STACK: tile buffer.  SRC_CARRIED: unused.
-  int32_t edge;  // 2 * (caller's op index) + child: where this edge's P slots sit in the caller's arrays; < 0: the edge
-                 // belongs to a record of the input snapshot, its P copies start at library slot ~edge
-};
-struct PlanOp {
-  int32_t node;
-  PlanChild ch[2];
-  int32_t out_buf;               // tiled kernel: shared-memory tile buffer of the result, or -1
-  int32_t pf_buf;                // tiled kernel: tile buffer a stored child is prefetched into, or -1
-  uint8_t is_root, keep, stream, spill, pushed;
-  uint8_t make_rec;              // not stored: the returned snapshot keeps the node as a record (small subtree)
-  uint8_t synthetic;             // not in the caller's list: a record of the input snapshot recomputed as a sibling
-};
-struct PlanLaunch { int r_begin, r_end, max_ops, n_bufs; };
-struct EvalPlan {
-  // key (full evaluations only)
-  int flags = 0, n_lists = 0, split_env = 0;
-  std::vector<int32_t> key_offsets, key_nodes, key_children;
-  // compiled form
-  std::vector<PlanOp> ops;
-  std::vector<RangeDesc> ranges;
-  std::vector<PlanLaunch> launches;
-  int64_t bytes_written = 0, bytes_read = 0;
-  int n_stored = 0, n_buffer_reads = 0, n_stack = 0, n_spills = 0, n_cherries = 0, n_small_recs = 0;
-  int n_inlined = 0;   // ops computed inside their parent's op (SRC_SMALL): in `ops` for their descriptor, in no range
-  uint64_t stamp = 0;
-};
-constexpr int PLAN_FLAG_MASK = CB_EVAL_WANT_SNAPSHOT | CB_EVAL_STORE_ROOT | CB_EVAL_FORCE_LEVELS | CB_EVAL_FORCE_WALK | CB_EVAL_NO_FOLD;
-constexpr int PLAN_CACHE_SIZE = 6;
-
 struct cb_ctx {
   int device = 0;
   cudaStream_t stream = nullptr;
@@ -245,11 +191,7 @@ struct cb_ctx {
   std::vector<void*> peer_opened;      // IPC mappings to close
   int32_t* d_comm_error = nullptr;
   unsigned long long epoch = 0;
-  // plans of full evaluations, cached per topology; scratch plan of dirty-path evaluations
-  std::vector<EvalPlan> plans;
-  EvalPlan scratch_plan;
-  uint64_t plan_clock = 0, plan_builds = 0;
-  bool no_plan_cache = false;
+  PlanCache plan_cache;
   std::vector<int> work_new_bufs, work_new_nodes, work_cherry_nodes;
   cudaEvent_t ev_main0 = nullptr, ev_main1 = nullptr;  // around the pruning launches proper (without pre-passes)
   double host_us[6] = {0, 0, 0, 0, 0, 0};  // accumulated per-evaluation host time: plan, fill, upload+launch, sync, bookkeeping, calls
@@ -333,7 +275,7 @@ static int create_impl(int device, cb_ctx** out) {
   if (getenv("CYBAYES_S2T_SMALL_RECS")) c->s2t_small_recs = atoi(getenv("CYBAYES_S2T_SMALL_RECS")) != 0;
   c->s2t_slots = c->s2t_minb == 4 ? 2 : c->s2t_minb == 3 ? 3 : 4;
   if (const char* v = getenv("CYBAYES_S2T_SLOTS")) c->s2t_slots = std::max(0, std::min(8, atoi(v)));
-  if (getenv("CYBAYES_NO_PLAN_CACHE")) c->no_plan_cache = true;
+  if (getenv("CYBAYES_NO_PLAN_CACHE")) c->plan_cache.no_plan_cache = true;
   if (const char* v = getenv("CYBAYES_MAX_DEVICE_BYTES")) c->max_dev_bytes = atoll(v);
 #define CB_S2T_ATTR(CC, MB, VV) CU(cudaFuncSetAttribute(prune_s2t_kernel<CC, MB, VV>, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024))
   CB_S2T_ATTR(4, 2, 1); CB_S2T_ATTR(4, 3, 1); CB_S2T_ATTR(1, 2, 1); CB_S2T_ATTR(1, 3, 1);   // + 384 B static each
@@ -354,7 +296,7 @@ static int create_impl(int device, cb_ctx** out) {
 }
 
 static void free_alignment(cb_ctx* c) {
-  c->plans.clear();
+  c->plan_cache.plans.clear();
   if (c->d_images) dev_free(c, c->d_images, (size_t)c->images_cap * sizeof(S2TImage));
   c->d_images = nullptr;
   c->images_cap = 0;
@@ -902,9 +844,14 @@ static LaunchConst make_const(cb_ctx* c) {
   return k;
 }
 
-constexpr int MAX_CHAIN_OPS = 4096;          // longer dirty paths fall back to the level schedule
-constexpr int64_t WALK_MIN_SITES_S2 = 32768; // below this a site tile cannot fill the GPU: use levels
-constexpr int64_t WALK_MIN_SITES_GENERAL = 32768;
+// What the planner needs to know of the context, including the launch geometry of the kernel the alignment runs on.
+static PlanConfig plan_config(const cb_ctx* c) {
+  const int64_t tile_sites = c->s2_tiled ? S2T_THREADS : c->family_s2 ? 256 * c->s2_vec : c->dmma_rc ? RC_T : c->use_dmma ? DM_T : GEN_T;
+  const int blocks_per_sm = c->s2_tiled ? c->s2t_minb : c->family_s2 ? (c->s2_vec == 1 ? 3 : 2) : c->dmma_rc ? 1 : 2;
+  return PlanConfig{c->n_taxa, c->n_cats, c->code_bytes, c->P, (int64_t)c->buffer_bytes, c->sm_count, c->family_s2,
+                    c->dmma_rc, c->s2_tiled, c->s2t_slots, c->s2t_bulk, c->s2t_prefetch, c->s2t_small_recs,
+                    c->s2_stream_stores, tile_sites, c->family_s2 ? 1 : c->n_cats, blocks_per_sm};
+}
 
 static int general_rows_per_chunk(int S) {
   // rows of the two P matrices staged per pass (multiple of 4, <= 64).  Prefer a footprint
@@ -1048,514 +995,6 @@ static int materialize_cherry(cb_ctx* c, const Snapshot& sn, int rec, int* buf_o
   return 0;
 }
 
-// ---- plans --------------------------------------------------------------------------------------------------
-// An evaluation is compiled into a PLAN: which ops run (cherries folded away), in which order, in which ranges
-// and launches, where every child comes from, which results are stored.  The plan of a FULL evaluation depends only
-// on the op list and the flags, so it is cached per topology (a handful of trees are alive at a time in an MCMC
-// run: the current one and the proposals); executing a cached plan only refills buffer pointers and P slots.
-//
-// Schedules (all run the same per-node arithmetic, so results are bit-identical):
-//   CHAIN  a dirty path: one launch, one block range walks the ops, the on-path partial is
-//          carried in registers / shared memory                        (ML_gamma.pyx:99-114)
-//   WALK   a whole (sub)tree in ONE launch; every block walks all ops for its site tile depth-first.  The child
-//          finished last is carried on chip; the other child of a node with two internal children is pushed on a
-//          stack in shared memory (tiled 2-state kernel: K tile buffers per warp) or, when the stack is full or the
-//          kernel has none, written to its buffer and read back.  The visiting order minimises those read-backs
-//          (dynamic programme over the tree; ties: heavier subtree first, so a read-back finds its line in L2).
-//   LEVELS one launch per tree level, grid.y = nodes of the level: the latency schedule for
-//          small alignments where a site tile alone cannot fill the GPU.
-enum Schedule { SCHED_CHAIN = 0, SCHED_WALK = 1, SCHED_LEVELS = 2 };
-
-
-static int build_plan(cb_ctx* c, const Snapshot* sin, int n_lists, const int32_t* offsets_in, const int32_t* nodes_in,
-                      const int32_t* children_in, int flags, EvalPlan& plan) {
-  const int N = c->n_taxa, n_nodes = 2 * N;  // ids 1 .. 2N-1
-  const bool fold = c->family_s2 && !(flags & CB_EVAL_NO_FOLD);
-  const bool want_snap = (flags & CB_EVAL_WANT_SNAPSHOT) != 0;
-  const bool store_root = (flags & CB_EVAL_STORE_ROOT) != 0;
-  const int C = c->n_cats;
-  const int K = c->s2_tiled ? c->s2t_slots : 0;  // stack slots of the kernel
-  const int slot_base = c->s2t_bulk ? S2T_STAGING : 0;  // tile buffers below it are the staging buffers of the bulk-store path
-  plan.ops.clear(); plan.ranges.clear(); plan.launches.clear();
-  plan.bytes_written = plan.bytes_read = 0;
-  plan.n_stored = plan.n_buffer_reads = plan.n_stack = plan.n_spills = plan.n_cherries = plan.n_small_recs = 0;
-  plan.n_inlined = 0;
-  const int64_t tip_row_bytes = c->P * c->code_bytes;
-  // small subtrees (children: tips / cherries) of a cache-kept pass are kept as records instead of being stored
-  const bool small_recs = c->s2_tiled && c->s2t_small_recs && want_snap;
-  auto snap_cherry = [&](int nd) {   // the input snapshot holds node nd as a record (a folded cherry or a small subtree)
-    return fold && sin && nd < (int)sin->cherry_of_node.size() && sin->cherry_of_node[nd] >= 0;
-  };
-
-  struct LOp { int32_t node, caller; int32_t child[2], folded[2]; };
-  std::vector<LOp> L;
-  std::vector<int32_t> parent_op(n_nodes), folded_at(n_nodes), op_of_node(n_nodes, -1);
-  std::vector<int> kid[2], n_sub, order, pos_of, range_id, push_slot, first_kid, level_of, by_level;
-  std::vector<std::pair<int, int>> segs;
-  std::vector<int> seg_of;     // op -> segment (0 = top / whole list, s + 1 = cut subtree s)
-  std::vector<int> f;          // DP table [op][k]
-  std::vector<char> read_back;
-  std::vector<int> small_of;   // op -> its child (0 / 1) that it computes itself (SRC_SMALL), or -1
-  std::vector<char> inlined;   // op -> computed inside its parent's op
-  bool single_launch = true;
-
-  for (int li = 0; li < n_lists; ++li) {
-    const int b_in = offsets_in[li], e_in = offsets_in[li + 1];
-    REQUIRE(e_in > b_in, "empty op list %d", li);
-    // ---- cherry folding (2-state family): an op whose two children are tips is not run: its parent (always in the
-    // list) takes it as a SRC_CHERRY child and looks the cherry's 3 x 3 possible partials up
-    L.clear();
-    std::fill(parent_op.begin(), parent_op.end(), -1);
-    std::fill(folded_at.begin(), folded_at.end(), -1);
-    for (int i = b_in; i < e_in; ++i)
-      for (int kx = 0; kx < 2; ++kx) {
-        const int ch = children_in[2 * i + kx];
-        REQUIRE((ch >= 1 && ch <= N) || (ch > N && ch < n_nodes), "op %d: bad child id %d", i, ch);
-        if (ch > N) parent_op[ch] = i;
-      }
-    for (int i = b_in; i < e_in; ++i) {
-      const int node = nodes_in[i], c0 = children_in[2 * i], c1 = children_in[2 * i + 1];
-      REQUIRE(node > N && node < n_nodes, "op %d: node %d is not an internal node", i, node);
-      const bool cherry = fold && c0 <= N && c1 <= N && i != e_in - 1 && parent_op[node] > i;
-      if (cherry) {
-        folded_at[node] = i;
-        plan.n_cherries++;
-        continue;
-      }
-      LOp o;
-      o.node = node;
-      o.caller = i;
-      for (int kx = 0; kx < 2; ++kx) {
-        const int ch = children_in[2 * i + kx];
-        o.child[kx] = ch;
-        o.folded[kx] = ch > N ? folded_at[ch] : -1;
-      }
-      L.push_back(o);
-    }
-    // Children that the input snapshot holds as records of small subtrees (not cherries) are recomputed here: one
-    // synthetic op each, placed before the caller's ops; the walk pushes / carries its result like any other child.
-    if (sin && c->s2_tiled) {
-      std::vector<LOp> syn;
-      auto is_rec = [&](int nd) { return nd > N && nd < (int)sin->cherry_of_node.size() && sin->cherry_of_node[nd] >= 0; };
-      for (const LOp& o : L)
-        for (int kx = 0; kx < 2; ++kx) {
-          const int ch = o.child[kx];
-          if (ch <= N || o.folded[kx] >= 0 || !is_rec(ch)) continue;
-          const CherryRec& r = c->recs[sin->cherry_of_node[ch]];
-          if (r.tip[0] <= N && r.tip[1] <= N) continue;   // a cherry: folded into the parent's table
-          bool in_list = false;
-          for (const LOp& q : L) in_list = in_list || q.node == ch;
-          if (in_list) continue;
-          LOp so;
-          so.node = ch;
-          so.caller = ~sin->cherry_of_node[ch];            // < 0: synthetic, names the record
-          so.child[0] = r.tip[0]; so.child[1] = r.tip[1];
-          so.folded[0] = so.folded[1] = -1;
-          syn.push_back(so);
-        }
-      if (!syn.empty()) L.insert(L.begin(), syn.begin(), syn.end());
-    }
-    const int n = (int)L.size();
-    // producers of the children inside this list (-1: tip, folded cherry or snapshot)
-    for (int j = 0; j < n; ++j) {
-      REQUIRE(op_of_node[L[j].node] < 0, "op %d: node %d is computed twice", L[j].caller, L[j].node);
-      op_of_node[L[j].node] = j;
-    }
-    auto cleanup = [&] { for (int j = 0; j < n; ++j) op_of_node[L[j].node] = -1; };
-    kid[0].assign(n, -1);
-    kid[1].assign(n, -1);
-    for (int j = 0; j < n; ++j)
-      for (int kx = 0; kx < 2; ++kx) {
-        const int ch = L[j].child[kx];
-        if (ch > N && L[j].folded[kx] < 0 && op_of_node[ch] >= 0) {
-          if (op_of_node[ch] >= j) { cleanup(); return fail("op %d: child %d is computed after its parent", L[j].caller, ch); }
-          kid[kx][j] = op_of_node[ch];
-        } else if (ch > N && L[j].folded[kx] < 0) {
-          const bool in_snap = sin && ch < (int)sin->buf_of_node.size() &&
-                               (sin->buf_of_node[ch] >= 0 || (ch < (int)sin->cherry_of_node.size() && sin->cherry_of_node[ch] >= 0));
-          if (!in_snap) { cleanup(); return fail("op %d: child %d is neither recomputed nor in the input snapshot", L[j].caller, ch); }
-        }
-      }
-    cleanup();
-    // chain: every op after the first consumes exactly the previous op and nothing else of the list
-    bool chain = !(flags & CB_EVAL_FORCE_LEVELS) && n <= MAX_CHAIN_OPS;
-    for (int j = 0; j < n && chain; ++j) {
-      const int a0 = kid[0][j], a1 = kid[1][j];
-      if (j == 0) chain = (a0 < 0 && a1 < 0);
-      else chain = (a0 == j - 1) != (a1 == j - 1) && (a0 < 0 || a0 == j - 1) && (a1 < 0 || a1 == j - 1);
-    }
-    Schedule sched = SCHED_CHAIN;
-    if (!chain) {
-      // the register-carried kernel only pays off when the partial is carried: its alignments always walk;
-      // candidates of a batch always walk (one range per candidate)
-      const bool big = c->dmma_rc || c->P >= (c->family_s2 ? WALK_MIN_SITES_S2 : WALK_MIN_SITES_GENERAL);
-      sched = ((big || n_lists > 1 || (flags & CB_EVAL_FORCE_WALK)) && !(flags & CB_EVAL_FORCE_LEVELS)) ? SCHED_WALK : SCHED_LEVELS;
-      if (n_lists > 1 && sched == SCHED_LEVELS) return fail("cb_eval_batch: candidate %d is not a chain (level schedule forced)", li);
-    }
-
-    // Tiled kernel: a (tip, cherry) subtree that is not stored is computed inside its parent's op (SRC_SMALL) when the
-    // parent runs in the same range and its other child is a tip or the op carried into it -- the same arithmetic
-    // without an op of its own (image, dispatch, rescale, loop iteration) and without a stack slot.
-    small_of.assign(n, -1);
-    inlined.assign(n, 0);
-    int n_inl = 0;
-    auto is_cherry = [&](int j, int kx) {   // the child resolves to SRC_CHERRY (below)
-      const int ch = L[j].child[kx];
-      return ch > N && (L[j].folded[kx] >= 0 || (kid[kx][j] < 0 && snap_cherry(ch)));
-    };
-    auto pick_small = [&] {
-      if (!c->s2_tiled) return;
-      for (int j = 0; j < n; ++j)
-        for (int kx = 1; kx >= 0 && small_of[j] < 0; --kx) {
-          const int s = kid[kx][j], o = kid[1 - kx][j];
-          if (s < 0 || seg_of[s] != seg_of[j]) continue;
-          const bool tip_cherry = (L[s].child[0] <= N && is_cherry(s, 1)) || (L[s].child[1] <= N && is_cherry(s, 0));
-          // not stored: likelihood-only pass, a recomputed record, or kept as a record (make_rec below; checked there)
-          const bool unstored = !want_snap || L[s].caller < 0 || small_recs;
-          const bool sibling_ok = L[j].child[1 - kx] <= N || (o >= 0 && seg_of[o] == seg_of[j]);
-          if (tip_cherry && unstored && sibling_ok) {
-            small_of[j] = kx;
-            inlined[s] = 1;
-            n_inl++;
-          }
-        }
-    };
-    order.resize(n);
-    for (int j = 0; j < n; ++j) order[j] = j;
-    seg_of.assign(n, 0);
-    push_slot.assign(n, -1);
-    segs.clear();
-    if (sched == SCHED_WALK) {
-      // subtree sizes in ops (children precede parents in the caller's order)
-      n_sub.assign(n, 1);
-      for (int j = 0; j < n; ++j)
-        for (int kx = 0; kx < 2; ++kx)
-          if (kid[kx][j] >= 0) n_sub[j] += n_sub[kid[kx][j]];
-      bool rooted = (n_sub[n - 1] == n);  // every op under the last one
-      if (!rooted) {
-        REQUIRE(n_lists == 1, "cb_eval_batch: candidate %d has ops that are not under its root", li);
-        sched = SCHED_LEVELS;
-      } else {
-        // When the alignment gives too few site tiles to fill the GPU for a whole sequential walk (small shards), the
-        // tree is cut into independent subtrees of at most `limit` ops that run as parallel ranges of a first launch;
-        // the ops above the cut follow in a second launch.
-        int limit = n + 1;
-        if (n_lists == 1) {
-          const int64_t tile_sites = c->s2_tiled ? S2T_THREADS : (c->family_s2 ? (int64_t)256 * c->s2_vec : (c->dmma_rc ? RC_T : (c->use_dmma ? DM_T : GEN_T)));
-          const int64_t blocks = (c->P + tile_sites - 1) / tile_sites * (c->family_s2 ? 1 : c->n_cats);
-          const int64_t slots = (int64_t)c->sm_count * (c->s2_tiled ? c->s2t_minb : (c->family_s2 ? (c->s2_vec == 1 ? 3 : 2) : (c->dmma_rc ? 1 : 2)));
-          // Every block walks the whole list (0.7 ms on C4, 3 ms on a C5 shard), so a ragged last wave is expensive even
-          // at many waves: 2-3 % at 8.8 waves, 12 % at 4.4 and 5.3.  Measured: C4 6.07 -> 5.91 ms on 1 GPU and 3.28 ->
-          // 2.98 ms per GPU on 2; the C5 shard of an 8-GPU run (25 000 patterns x 64 states) 17.7 -> 15.9 ms.
-          // Under one wave the cut is there for parallelism (about 8 waves of ranges); from one wave up it only has to
-          // even out the tail, and a small limit costs more in the launch of the ops above the cut (16 ops at limit 93
-          // on a 125 000-pattern shard: 65 us of 800) than it gains: a third of the tree per range measured best there
-          // (0.794 -> 0.77 ms).
-          if (blocks < 16 * slots && n >= 64 && !(flags & CB_EVAL_FORCE_WALK)) {
-            int lim = (int)(n * blocks / (8 * slots)) + 1;
-            if (blocks >= slots) lim = std::max(lim, n / 3);
-            limit = std::max(16, std::min(256, lim));
-          }
-          if (plan.split_env > 0) limit = std::max(2, plan.split_env);
-          if (limit >= n) limit = n + 1;  // nothing to cut
-        }
-        std::vector<int> cut, top, stack;
-        if (limit <= n) {
-          // walk down from the root: ops with a subtree above the limit stay in the top segment
-          stack.push_back(n - 1);
-          while (!stack.empty()) {
-            const int j = stack.back();
-            stack.pop_back();
-            if (n_sub[j] <= limit) { cut.push_back(j); continue; }
-            for (int kx = 0; kx < 2; ++kx)
-              if (kid[kx][j] >= 0) stack.push_back(kid[kx][j]);
-          }
-          std::stable_sort(cut.begin(), cut.end(), [&](int x, int y) { return n_sub[x] > n_sub[y]; });  // big first
-          // segment membership: everything under a cut root belongs to that root's segment
-          for (size_t s = 0; s < cut.size(); ++s) {
-            stack.push_back(cut[s]);
-            while (!stack.empty()) {
-              const int j = stack.back();
-              stack.pop_back();
-              seg_of[j] = (int)s + 1;
-              for (int kx = 0; kx < 2; ++kx)
-                if (kid[kx][j] >= 0) stack.push_back(kid[kx][j]);
-            }
-          }
-        }
-        pick_small();
-        // children the walk visits: a cut root lives in another launch and is read from its buffer; an inlined subtree
-        // is computed by its parent, like a tip
-        auto walk_kid = [&](int kx, int j) {
-          const int a = kid[kx][j];
-          return a >= 0 && seg_of[a] == seg_of[j] && !inlined[a] ? a : -1;
-        };
-        // visiting order per segment: f[j][k] = fewest read-backs in j's subtree (inside its segment) with k free stack
-        // slots; of two internal children the first visited is pushed (or read back when k == 0), the second carried
-        f.assign((size_t)n * (K + 1), 0);
-        first_kid.assign((size_t)n * (K + 1), 0);
-        for (int j = 0; j < n; ++j) {
-          const int a = walk_kid(0, j), b2 = walk_kid(1, j);
-          for (int kk = 0; kk <= K; ++kk) {
-            int& fj = f[(size_t)j * (K + 1) + kk];
-            if (a >= 0 && b2 >= 0) {
-              const int k1 = kk > 0 ? kk - 1 : 0, miss = kk == 0 ? 1 : 0;
-              const int ca = f[(size_t)a * (K + 1) + kk] + miss + f[(size_t)b2 * (K + 1) + k1];
-              const int cb2 = f[(size_t)b2 * (K + 1) + kk] + miss + f[(size_t)a * (K + 1) + k1];
-              const bool a_first = ca < cb2 || (ca == cb2 && n_sub[a] >= n_sub[b2]);
-              fj = a_first ? ca : cb2;
-              first_kid[(size_t)j * (K + 1) + kk] = a_first ? 0 : 1;
-              // third choice: read the first child back although a slot is free, so that the second keeps all kk slots
-              // (one read-back here instead of one at every fork of a subtree left with too few slots)
-              const int cs = f[(size_t)a * (K + 1) + kk] + 1 + f[(size_t)b2 * (K + 1) + kk];
-              if (kk > 0 && cs < fj) {
-                fj = cs;
-                first_kid[(size_t)j * (K + 1) + kk] = (n_sub[a] >= n_sub[b2] ? 0 : 1) | 2;
-              }
-            } else if (a >= 0) {
-              fj = f[(size_t)a * (K + 1) + kk];
-            } else if (b2 >= 0) {
-              fj = f[(size_t)b2 * (K + 1) + kk];
-            }
-          }
-        }
-        std::vector<int> out;
-        out.reserve(n);
-        struct Frame { int j, k, phase; };
-        std::vector<Frame> fr;
-        auto emit = [&](int root_op) {
-          fr.push_back({root_op, K, 0});
-          while (!fr.empty()) {
-            Frame& t = fr.back();
-            const int j = t.j, kk = t.k;
-            const int a = walk_kid(0, j), b2 = walk_kid(1, j);
-            if (a >= 0 && b2 >= 0) {
-              const int fk = first_kid[(size_t)j * (K + 1) + kk];
-              const bool push = kk > 0 && !(fk & 2);
-              const int x = (fk & 1) == 0 ? a : b2, y = (fk & 1) == 0 ? b2 : a;
-              if (t.phase == 0) { t.phase = 1; fr.push_back({x, kk, 0}); continue; }
-              if (t.phase == 1) {
-                push_slot[x] = push ? slot_base + (K - kk) : -1;
-                t.phase = 2;
-                fr.push_back({y, push ? kk - 1 : kk, 0});
-                continue;
-              }
-            } else if (a >= 0 || b2 >= 0) {
-              if (t.phase == 0) { t.phase = 2; fr.push_back({a >= 0 ? a : b2, kk, 0}); continue; }
-            }
-            out.push_back(j);
-            fr.pop_back();
-          }
-        };
-        if (limit > n) {
-          emit(n - 1);
-        } else {
-          for (int r : cut) {
-            const int b0 = (int)out.size();
-            emit(r);
-            segs.push_back({b0, (int)out.size()});
-          }
-          emit(n - 1);
-        }
-        REQUIRE((int)out.size() == n - n_inl, "internal error: walk order covers %d of %d ops", (int)out.size(), n - n_inl);
-        for (int j = 0; j < n; ++j)
-          if (inlined[j]) out.push_back(j);   // descriptors only: after the ops the ranges run
-        order = out;
-      }
-    } else if (sched == SCHED_CHAIN) {
-      pick_small();   // only the first op of a chain can be such a subtree; its parent takes it beside a tip
-      if (n_inl > 0) {
-        std::stable_partition(order.begin(), order.end(), [&](int j) { return !inlined[j]; });
-      }
-    }
-    const int n_exec = n - n_inl;   // positions [n_exec, n): inlined ops
-    plan.n_inlined += n_inl;
-    pos_of.assign(n, 0);
-    for (int p = 0; p < n; ++p) pos_of[order[p]] = p;
-    range_id.assign(n, 0);   // by position
-    for (size_t si = 0; si < segs.size(); ++si)
-      for (int p = segs[si].first; p < segs[si].second; ++p) range_id[p] = (int)si + 1;
-    // launch of a position: split walk = cut segments first (0), top second (1); levels: see below
-    auto same_range = [&](int p0, int p1) { return sched != SCHED_LEVELS && range_id[p0] == range_id[p1]; };
-
-    // where does each child come from; which ops are read back from memory by a later op?
-    read_back.assign(n, 0);
-    const int base = (int)plan.ops.size();
-    plan.ops.resize(base + n);
-    int staging_rr = 0;
-    for (int p = 0; p < n; ++p) {
-      const int j = order[p];
-      PlanOp& po = plan.ops[base + p];
-      po.node = L[j].node;
-      po.is_root = (j == n - 1);
-      REQUIRE(!po.is_root || p == n_exec - 1, "internal error: root is not last");
-      po.keep = po.stream = po.spill = po.pushed = po.make_rec = 0;
-      po.synthetic = L[j].caller < 0 ? 1 : 0;
-      po.out_buf = po.pf_buf = -1;
-      for (int kx = 0; kx < 2; ++kx) {
-        PlanChild& pc = po.ch[kx];
-        const int ch = L[j].child[kx];
-        pc.edge = L[j].caller >= 0 ? 2 * L[j].caller + kx : ~((~L[j].caller) * 2 * C + kx * C);
-        if (ch <= N) {
-          pc.kind = SRC_TIP;
-          pc.ref = ch;
-          plan.bytes_read += tip_row_bytes;
-        } else if (L[j].folded[kx] >= 0) {
-          pc.kind = SRC_CHERRY;
-          pc.ref = L[j].folded[kx];
-          plan.bytes_read += 2 * tip_row_bytes;
-        } else if (small_of[j] == kx) {
-          pc.kind = SRC_SMALL;
-          pc.ref = base + pos_of[kid[kx][j]];   // its descriptor
-        } else if (kid[kx][j] >= 0) {
-          const int jj = kid[kx][j], pp = pos_of[jj];
-          if (same_range(pp, p) && pp == p - 1) {
-            pc.kind = SRC_CARRIED;
-            pc.ref = 0;
-          } else if (same_range(pp, p) && push_slot[jj] >= 0) {
-            pc.kind = SRC_STACK;
-            pc.ref = push_slot[jj];
-            plan.n_stack++;
-          } else {
-            REQUIRE(pp < p, "internal error: producer of node %d runs after its consumer", ch);
-            pc.kind = SRC_BUFFER;
-            pc.ref = base + pp;
-            read_back[jj] = same_range(pp, p) ? 2 : 1;   // 2: inside one launch (a spill)
-            plan.bytes_read += (int64_t)c->buffer_bytes;
-            plan.n_buffer_reads++;
-          }
-        } else {
-          const bool rec = snap_cherry(ch);
-          pc.kind = rec ? SRC_CHERRY : SRC_BUFFER;
-          pc.ref = ~ch;
-          plan.bytes_read += rec ? 2 * tip_row_bytes : (int64_t)c->buffer_bytes;
-          if (!rec) plan.n_buffer_reads++;
-        }
-      }
-    }
-    plan.bytes_read += c->P * 8;  // pattern weights at the root
-    if (c->s2_tiled)  // the tiled kernel wants the children in canonical order (products and exponent sums commute exactly)
-      for (int p = 0; p < n; ++p) {
-        PlanOp& po = plan.ops[base + p];
-        if (s2t_rank(po.ch[1].kind) < s2t_rank(po.ch[0].kind)) std::swap(po.ch[0], po.ch[1]);
-        REQUIRE(s2t_combo(po.ch[0].kind, po.ch[1].kind) >= 0, "internal error: op of node %d has children of kinds %d, %d", po.node,
-                po.ch[0].kind, po.ch[1].kind);
-      }
-    for (int p = 0; p < n; ++p) {
-      const int j = order[p];
-      PlanOp& po = plan.ops[base + p];
-      po.keep = po.is_root ? (want_snap && store_root) : ((want_snap && !po.synthetic) || read_back[j] != 0);
-      po.stream = (po.keep && read_back[j] == 0 && c->s2_stream_stores) ? 1 : 0;
-      po.spill = (read_back[j] == 2) ? 1 : 0;
-      if (po.keep) {
-        plan.bytes_written += (int64_t)c->buffer_bytes;
-        plan.n_stored++;
-        if (po.spill) plan.n_spills++;
-      }
-      // small subtrees (children: tips / cherries) are not stored: the returned snapshot keeps a record
-      if (small_recs && po.keep && !po.is_root && !po.synthetic && read_back[j] == 0 &&
-          (po.ch[0].kind == SRC_TIP || po.ch[0].kind == SRC_CHERRY) && po.ch[1].kind == SRC_CHERRY) {
-        po.keep = 0;
-        po.stream = 0;
-        po.make_rec = 1;
-        plan.bytes_written -= (int64_t)c->buffer_bytes;
-        plan.n_stored--;
-        plan.n_small_recs++;
-      }
-      // an inlined op has no store of its own: a buffer given to it would enter the snapshot unwritten
-      REQUIRE(!inlined[j] || !po.keep, "internal error: inlined node %d would be stored", po.node);
-      if (c->s2_tiled) {
-        if (push_slot[j] >= 0 && !po.is_root) { po.out_buf = push_slot[j]; po.pushed = 1; }
-        else if (c->s2t_bulk && po.keep && !po.spill) { po.out_buf = staging_rr; staging_rr ^= 1; }
-      }
-    }
-    int max_slot = -1;
-    for (int j = 0; j < n; ++j) max_slot = std::max(max_slot, push_slot[j]);
-    if (c->s2_tiled && c->s2t_prefetch && max_slot < 2 && !c->s2t_bulk) {
-      // Dirty paths and other lists with a shallow stack: a stored partial that comes from the input snapshot (or an
-      // earlier launch) and is read beside a carried child is prefetched into a tile buffer two ops ahead (three rotating
-      // buffers above the stack slots in use) and then read like a stack slot: the path keeps three sibling tiles per
-      // warp in flight instead of exposing one DRAM latency per op.
-      const int pf_base = max_slot + 1;
-      int rr = 0;
-      for (int p = 0; p < n; ++p) {
-        PlanOp& po = plan.ops[base + p];
-        if (po.ch[0].kind != SRC_CARRIED || po.ch[1].kind != SRC_BUFFER) continue;
-        const int ref = po.ch[1].ref;
-        const bool other_launch = ref < 0 || !same_range(ref - base, p);
-        if (!other_launch) continue;
-        po.ch[1].kind = SRC_STACK;     // read from the tile buffer; po.ch[1].ref keeps naming the stored partial
-        po.pf_buf = pf_base + rr;
-        rr = (rr + 1) % 3;
-      }
-    }
-
-    // ranges and launches
-    auto bufs_of = [&](int p0, int p1) {
-      int nb = 0;
-      for (int p = p0; p < p1; ++p) {
-        const PlanOp& po = plan.ops[base + p];
-        nb = std::max(nb, std::max(po.out_buf, po.pf_buf) + 1);
-        for (int kx = 0; kx < 2; ++kx)
-          if (po.ch[kx].kind == SRC_STACK && po.pf_buf < 0) nb = std::max(nb, po.ch[kx].ref + 1);
-      }
-      return nb;
-    };
-    if (sched == SCHED_WALK && !segs.empty()) {
-      single_launch = false;
-      const int start = (int)plan.ranges.size();
-      int mx = 1, nb = 0;
-      for (auto& sg : segs) {
-        plan.ranges.push_back(RangeDesc{base + sg.first, base + sg.second, -1, 0});
-        mx = std::max(mx, sg.second - sg.first);
-        nb = std::max(nb, bufs_of(sg.first, sg.second));
-      }
-      plan.launches.push_back({start, (int)plan.ranges.size(), mx, nb});
-      const int tb = segs.back().second;
-      plan.ranges.push_back(RangeDesc{base + tb, base + n_exec, li, 0});
-      plan.launches.push_back({(int)plan.ranges.size() - 1, (int)plan.ranges.size(), n_exec - tb, bufs_of(tb, n_exec)});
-    } else if (sched != SCHED_LEVELS) {
-      plan.ranges.push_back(RangeDesc{base, base + n_exec, li, 0});
-    } else {
-      single_launch = false;
-      level_of.assign(n, 1);
-      int max_level = 1;
-      for (int j = 0; j < n; ++j) {
-        int lv = 1;
-        for (int kx = 0; kx < 2; ++kx)
-          if (kid[kx][j] >= 0) lv = std::max(lv, level_of[kid[kx][j]] + 1);
-        level_of[j] = lv;
-        max_level = std::max(max_level, lv);
-      }
-      by_level.resize(n);
-      for (int j = 0; j < n; ++j) by_level[j] = j;
-      std::stable_sort(by_level.begin(), by_level.end(), [&](int x, int y) { return level_of[x] < level_of[y]; });
-      int pos = 0;
-      for (int lv = 1; lv <= max_level; ++lv) {
-        const int start = (int)plan.ranges.size();
-        int nb = 0;
-        while (pos < n && level_of[by_level[pos]] == lv) {
-          const int j = by_level[pos++];   // order is the identity for this schedule
-          plan.ranges.push_back(RangeDesc{base + j, base + j + 1, (j == n - 1) ? li : -1, 0});
-          nb = std::max(nb, bufs_of(j, j + 1));
-        }
-        if ((int)plan.ranges.size() > start) plan.launches.push_back({start, (int)plan.ranges.size(), 1, nb});
-      }
-    }
-  }
-  if (single_launch) {
-    int mx = 0, nb = 0;
-    for (const RangeDesc& r : plan.ranges) mx = std::max(mx, r.end - r.begin);
-    for (const PlanOp& po : plan.ops) {
-      nb = std::max(nb, std::max(po.out_buf, po.pf_buf) + 1);
-      for (int kx = 0; kx < 2; ++kx)
-        if (po.ch[kx].kind == SRC_STACK && po.pf_buf < 0) nb = std::max(nb, po.ch[kx].ref + 1);
-    }
-    plan.launches.push_back({0, (int)plan.ranges.size(), mx, nb});
-  }
-  return 0;
-}
-
 // Releases what an evaluation acquired when it fails part-way (buffers and cherry records go back to their pools).
 struct EvalGuard {
   cb_ctx* c;
@@ -1584,44 +1023,9 @@ static int eval_impl(cb_ctx* c, int snapshot_in, int n_lists, const int32_t* off
 
   const double t_begin = now_us();
   // ---- the plan: cached per (op list, flags) for full evaluations, built on the spot for dirty paths
-  const int split_env = getenv("CYBAYES_WALK_SPLIT") ? atoi(getenv("CYBAYES_WALK_SPLIT")) : 0;
-  EvalPlan* plan = nullptr;
-  if (snapshot_in < 0 && !c->no_plan_cache) {
-    for (auto& p : c->plans)
-      if (p.n_lists == n_lists && p.flags == (flags & PLAN_FLAG_MASK) && p.split_env == split_env &&
-          (int)p.key_nodes.size() == total_in && memcmp(p.key_offsets.data(), offsets_in, (size_t)(n_lists + 1) * 4) == 0 &&
-          memcmp(p.key_nodes.data(), nodes_in, (size_t)total_in * 4) == 0 &&
-          memcmp(p.key_children.data(), children_in, (size_t)total_in * 8) == 0) {
-        plan = &p;
-        break;
-      }
-    if (!plan) {
-      if ((int)c->plans.size() < PLAN_CACHE_SIZE) {
-        c->plans.emplace_back();
-        plan = &c->plans.back();
-      } else {  // evict the least recently used
-        plan = &c->plans[0];
-        for (auto& p : c->plans)
-          if (p.stamp < plan->stamp) plan = &p;
-      }
-      plan->n_lists = 0;  // invalid while it is rebuilt
-      plan->split_env = split_env;
-      if (build_plan(c, nullptr, n_lists, offsets_in, nodes_in, children_in, flags, *plan)) { plan->key_nodes.clear(); return 1; }
-      plan->n_lists = n_lists;
-      plan->flags = flags & PLAN_FLAG_MASK;
-      plan->key_offsets.assign(offsets_in, offsets_in + n_lists + 1);
-      plan->key_nodes.assign(nodes_in, nodes_in + total_in);
-      plan->key_children.assign(children_in, children_in + 2 * (size_t)total_in);
-      c->plan_builds++;
-    }
-    plan->stamp = ++c->plan_clock;
-  } else {
-    plan = &c->scratch_plan;
-    plan->split_env = split_env;
-    if (build_plan(c, snapshot_in >= 0 ? &c->snaps[snapshot_in] : nullptr, n_lists, offsets_in, nodes_in, children_in, flags, *plan))
-      return 1;
-    c->plan_builds++;
-  }
+  const Snapshot* sin = snapshot_in >= 0 ? &c->snaps[snapshot_in] : nullptr;
+  const EvalPlan* plan = plan_for(c->plan_cache, plan_config(c), sin, c->recs, n_lists, offsets_in, nodes_in, children_in, flags);
+  if (!plan) return 1;
   const int total_ops = (int)plan->ops.size();
   const int n_ranges = (int)plan->ranges.size();
 
@@ -1634,7 +1038,6 @@ static int eval_impl(cb_ctx* c, int snapshot_in, int n_lists, const int32_t* off
   const double t_planned = now_us();
 
   // ---- fill the descriptors: buffers, pointers, P slots
-  const Snapshot* sin = snapshot_in >= 0 ? &c->snaps[snapshot_in] : nullptr;
   EvalGuard guard{c};
   std::vector<int>& new_bufs = c->work_new_bufs;
   std::vector<int>& new_nodes = c->work_new_nodes;

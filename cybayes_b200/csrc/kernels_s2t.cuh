@@ -13,7 +13,7 @@
 //   * Walk with a stack in shared memory.  A warp walks the whole op range for its tile depth-first.  The
 //     child finished last is carried in registers (as before); the other child of a node with two internal
 //     children is PUSHED into one of K tile buffers in shared memory and popped by its parent -- it is never
-//     read back from L2/HBM.  The host orders the walk (dynamic programme over the tree, cybayes_b200.cu) so
+//     read back from L2/HBM.  The host orders the walk (dynamic programme over the tree, plan.cpp) so
 //     that almost every such child fits the K slots (C4: 1 of 210 misses with K = 4, 31 with K = 3); the
 //     misses ("spills") go through global memory with plain stores/loads.  In steady state the kernel issues
 //     NO register-destination global loads: the tip codes (1 byte per site and tip) arrive in shared memory through
@@ -30,13 +30,11 @@
 
 namespace cb {
 
-constexpr int S2T_W = 32;          // sites per tile
-constexpr int S2T_WARPS = 8;       // tiles per block (a warp owns V consecutive tiles: 8 / V warps per block)
-constexpr int S2T_THREADS = S2T_W * S2T_WARPS;
+// the tile geometry (S2T_W, ...) and the canonical child order (s2t_rank, s2t_combo) are in cb_types.cuh: the planner
+// uses them too
 constexpr int S2T_RING_OPS = 4;    // op images per ring chunk
 __host__ __device__ constexpr int s2t_ring_stages(int minb) { return minb >= 3 ? 3 : 4; }  // chunks in the ring: a refill has
                                                                                          // (stages - 1) chunks of slack
-constexpr int S2T_STAGING = 2;     // bulk-store path only: tile buffers 0..1 per warp rotate as store staging, stack slots follow
 
 __host__ __device__ constexpr int s2t_tile_bytes(int C) { return S2T_W * (2 * C * 8 + 4); }
 
@@ -59,31 +57,10 @@ struct S2TImage {
 };
 static_assert(sizeof(S2TImage) == 1408, "S2TImage must stay 1408 bytes (a multiple of 16)");
 
-// Children of an op are kept in a canonical order (products and exponent sums commute exactly), which leaves twelve
-// possible pairs of child kinds; each has its own straight-line op body in the kernel.
-//
-// An inlined (tip, cherry) subtree (SRC_SMALL) is always child 1, beside a carried child or a tip.  Its op image holds
-// three children's worth of tables: tab[0] = child 0's P rows (4C doubles), the parent's P rows for the subtree (4C),
-// the subtree's P rows for its tip (4C); tab[1] = the subtree's cherry table.  Code rows: [0] child 0's tip, [1] the
-// subtree's tip, [2] and [3] the tips of its cherry.
-__host__ __device__ constexpr int s2t_rank(int kind) {
-  return kind == SRC_CARRIED ? 0 : kind == SRC_STACK ? 1 : kind == SRC_BUFFER ? 2 : kind == SRC_TIP ? 3 : kind == SRC_CHERRY ? 4 : 5;
-}
-enum S2TCombo : int32_t {
-  S2T_CARRIED_STACK = 0, S2T_CARRIED_BUFFER, S2T_CARRIED_TIP, S2T_CARRIED_CHERRY, S2T_BUFFER_BUFFER, S2T_BUFFER_TIP,
-  S2T_BUFFER_CHERRY, S2T_TIP_TIP, S2T_TIP_CHERRY, S2T_CHERRY_CHERRY, S2T_CARRIED_SMALL, S2T_TIP_SMALL, S2T_N_COMBOS
-};
 // does an op whose children have kinds k0, k1 (canonical order) read code row q of its image?
 __host__ __device__ inline bool s2t_row_used(int k0, int k1, int q) {
   return q == 0 ? (k0 == SRC_TIP || k0 == SRC_CHERRY) : q == 1 ? (k0 == SRC_CHERRY || k1 == SRC_SMALL)
                                                                : (k1 == SRC_CHERRY || k1 == SRC_SMALL || (q == 2 && k1 == SRC_TIP));
-}
-__host__ __device__ inline int s2t_combo(int k0, int k1) {   // kinds in canonical order; -1: not a pair the walk produces
-  if (k0 == SRC_CARRIED) return k1 == SRC_STACK ? S2T_CARRIED_STACK : k1 == SRC_BUFFER ? S2T_CARRIED_BUFFER : k1 == SRC_TIP ? S2T_CARRIED_TIP : k1 == SRC_CHERRY ? S2T_CARRIED_CHERRY : k1 == SRC_SMALL ? S2T_CARRIED_SMALL : -1;
-  if (k0 == SRC_BUFFER) return k1 == SRC_BUFFER ? S2T_BUFFER_BUFFER : k1 == SRC_TIP ? S2T_BUFFER_TIP : k1 == SRC_CHERRY ? S2T_BUFFER_CHERRY : -1;
-  if (k0 == SRC_TIP) return k1 == SRC_TIP ? S2T_TIP_TIP : k1 == SRC_CHERRY ? S2T_TIP_CHERRY : k1 == SRC_SMALL ? S2T_TIP_SMALL : -1;
-  if (k0 == SRC_CHERRY) return k1 == SRC_CHERRY ? S2T_CHERRY_CHERRY : -1;
-  return -1;
 }
 // how the result of an op leaves the registers
 enum S2TStore : int32_t {
