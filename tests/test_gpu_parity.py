@@ -95,7 +95,10 @@ def test_golden_full_and_dirty(name, golden_cases, gpu_backend):
     assert l3 == lnl
 
 
-def _random_problem(seed, n_taxa, n_sites, S, n_cats=4, missing=0.1, poly=0.02, bl_mean=0.1, n_poly=3):
+def _random_problem(seed, n_taxa, n_sites, S, n_cats=4, missing=0.1, poly=0.02, bl_mean=0.1, n_poly=3, code_dtype=None):
+    """Seeded tree, codes, ambiguity sets, pi, exchangeabilities and category rates.  Every category count above 1
+    gets the distinct discrete-Gamma rates of alpha = 0.7, so a kernel that mixes up categories gives another lnL.
+    code_dtype: np.uint16 forces 2-byte codes where 1 byte would do."""
     rng = np.random.default_rng(seed)
     pyr = random.Random(seed)
     # random topology: join two random subtrees until one is left; ids like the reference
@@ -123,10 +126,10 @@ def _random_problem(seed, n_taxa, n_sites, S, n_cats=4, missing=0.1, poly=0.02, 
     if len(amb) > 1:
         m = rng.random((n_taxa, n_sites)) < poly
         codes[m] = S + rng.integers(1, len(amb), size=int(m.sum()))
-    codes = codes.astype(np.uint8 if S + len(amb) <= 256 else np.uint16)
+    codes = codes.astype(code_dtype or (np.uint8 if S + len(amb) <= 256 else np.uint16))
     pi = rng.dirichlet(np.full(S, 5.0))
     er = rng.dirichlet(np.ones(S * (S - 1) // 2))
-    rates = oracle.site_rates(0.7, n_cats) if n_cats == 4 else [1.0] * n_cats
+    rates = oracle.site_rates(0.7, n_cats) if n_cats > 1 else [1.0]
     return tree, root, edges, codes, amb, pi, er, rates
 
 
