@@ -25,12 +25,14 @@ CHAIN_RELEASE_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_int)
 CHAIN_RATES_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_double, c_f64p)
 CHAIN_BETA_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, c_f64p, C.c_int, c_f64p)
 CHAIN_EIG_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, c_f64p, c_f64p, c_f64p)
+CHAIN_EVAL_SITES_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_int, C.c_int, c_i32p, c_i32p, c_i32p, c_f64p, C.c_int,
+                                  C.POINTER(C.c_int), c_f64p, c_f64p, c_f64p)
 
 
 class ChainBackend(C.Structure):
     _fields_ = [("user", C.c_void_p), ("pmat_build", CHAIN_BUILD_FN), ("eval", CHAIN_EVAL_FN),
                 ("snapshot_release", CHAIN_RELEASE_FN), ("site_rates", CHAIN_RATES_FN), ("f81_beta", CHAIN_BETA_FN),
-                ("gtr_eig", CHAIN_EIG_FN)]
+                ("gtr_eig", CHAIN_EIG_FN), ("eval_sites", CHAIN_EVAL_SITES_FN)]
 
 
 # name -> (restype, argtypes); mirrors include/cybayes_b200.h one to one
@@ -44,6 +46,7 @@ SIGNATURES = {
     "cb_chain_run": (C.c_int, [C.c_void_p, C.c_int64, c_i8p, c_i8p, c_f64p, c_f64p, c_f64p, c_f64p]),
     "cb_chain_get_state": (C.c_int, [C.c_void_p, c_i32p, c_i32p, c_f64p, c_f64p, c_f64p, c_f64p, c_f64p, c_f64p]),
     "cb_chain_counters": (C.c_int, [C.c_void_p, c_i64p, c_i64p]),
+    "cb_chain_site_lnl": (C.c_int, [C.c_void_p, c_f64p, c_f64p]),
     "cb_chain_destroy": (C.c_int, [C.c_void_p]),
     "cb_last_error": (C.c_char_p, []),
     "cb_version": (C.c_int, []),
@@ -61,6 +64,8 @@ SIGNATURES = {
     "cb_pmat_build": (C.c_int, [C.c_void_p, C.c_int, c_f64p, C.c_double, c_f64p, C.c_int, c_i32p, c_f64p, c_f64p]),
     "cb_eval": (C.c_int, [C.c_void_p, C.c_int, C.c_int, c_i32p, c_i32p, c_i32p, c_f64p, C.c_int,
                           C.POINTER(C.c_int), c_f64p]),
+    "cb_eval_sites": (C.c_int, [C.c_void_p, C.c_int, C.c_int, c_i32p, c_i32p, c_i32p, c_f64p, C.c_int,
+                                C.POINTER(C.c_int), c_f64p, c_f64p, c_f64p]),
     "cb_eval_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_int, c_i32p, c_i32p, c_i32p, c_i32p, c_f64p, c_f64p]),
     "cb_result_wait": (C.c_int, [C.c_void_p, c_f64p]),
     "cb_snapshot_retain": (C.c_int, [C.c_void_p, C.c_int]),

@@ -82,6 +82,9 @@ struct LaunchConst {
   struct Mail* mailbox;                // this rank's mailbox [2][CB_MB_OUTS][n_ranks]
   struct Mail* const* peer_mailbox;    // device array: every rank's mailbox (peer pointers opened through CUDA IPC)
   int32_t* comm_error;                 // set when a peer never delivered (timeout)
+  // Per-site output of the root epilogues (cb_eval_sites); both null in every other evaluation.
+  double* site_lnl;                    // [P]: log(sum_c pi.L_c,p / n_cats) + e_p ln 2, the term the reduction sums
+  double* site_post;                   // [C][P] or null: the category terms pi.L_c,p / n_cats the epilogue adds into s_p
 };
 
 // ---- tiled 2-state kernel (kernels_s2t.cuh): tile geometry and the child kinds its op bodies take

@@ -174,6 +174,8 @@ struct cb_ctx {
   double* d_root_dot = nullptr;
   int32_t* d_root_exp = nullptr;
   int out_cap = 0, max_blocks = 0;
+  double* d_site_lnl = nullptr;   // [P], cb_eval_sites only (allocated on first use)
+  double* d_site_post = nullptr;  // [C][P], cb_eval_sites with category posteriors only
   int last_n_out = 0;
   // scratch for pmat builds
   void* d_scratch = nullptr;
@@ -332,6 +334,9 @@ static void free_alignment(cb_ctx* c) {
   c->d_root_exp = nullptr;
   c->h_results = nullptr;
   c->out_cap = 0;
+  if (c->d_site_lnl) dev_free(c, c->d_site_lnl, (size_t)c->P * 8);
+  if (c->d_site_post) dev_free(c, c->d_site_post, (size_t)c->n_cats * c->P * 8);
+  c->d_site_lnl = c->d_site_post = nullptr;
 }
 
 extern "C" int cb_destroy(cb_ctx* c) {
@@ -841,6 +846,8 @@ static LaunchConst make_const(cb_ctx* c) {
   k.mailbox = nullptr;
   k.peer_mailbox = nullptr;
   k.comm_error = nullptr;
+  k.site_lnl = nullptr;
+  k.site_post = nullptr;
   return k;
 }
 
@@ -1007,10 +1014,11 @@ struct EvalGuard {
   }
 };
 
-// Shared implementation of cb_eval (n_lists = 1) and cb_eval_batch.
+// Shared implementation of cb_eval (n_lists = 1), cb_eval_batch and cb_eval_sites.  d_site_lnl / d_site_post: device
+// arrays the root epilogue fills per site (cb_eval_sites), else null.
 static int eval_impl(cb_ctx* c, int snapshot_in, int n_lists, const int32_t* offsets_in, const int32_t* nodes_in,
                      const int32_t* children_in, const int32_t* pslots_in, const double* pi, int flags,
-                     int* snapshot_out, double* lnl_out) {
+                     int* snapshot_out, double* lnl_out, double* d_site_lnl = nullptr, double* d_site_post = nullptr) {
   REQUIRE(c && c->n_states > 0, "cb_set_tips must come first");
   REQUIRE(offsets_in && nodes_in && children_in && pslots_in && pi, "null argument");
   REQUIRE(snapshot_in < 0 || snapshot_valid(c, snapshot_in), "invalid snapshot %d", snapshot_in);
@@ -1177,6 +1185,8 @@ static int eval_impl(cb_ctx* c, int snapshot_in, int n_lists, const int32_t* off
   LaunchConst k = make_const(c);
   k.ranges = reinterpret_cast<const RangeDesc*>(c->d_stage + off_ranges);
   k.pi = reinterpret_cast<const double*>(c->d_stage + off_pi);
+  k.site_lnl = d_site_lnl;
+  k.site_post = d_site_post;
   // Sharded over GPUs: the root kernel all-reduces the shard sums itself over peer memory (batches beyond CB_MB_OUTS
   // results: ncclAllReduce).  Either way without NCCL in the step the kernel writes lnL straight into mapped host
   // memory: no device -> host copy.
@@ -1305,6 +1315,44 @@ extern "C" int cb_eval_batch(cb_ctx* c, int snapshot_in, int n_batch, const int3
                              const int32_t* children, const int32_t* pslots, const double* pi, double* lnl_out) {
   REQUIRE(n_batch >= 1, "empty batch");
   return guarded([&] { return eval_impl(c, snapshot_in, n_batch, op_offsets, nodes, children, pslots, pi, 0, nullptr, lnl_out); });
+}
+
+extern "C" int cb_eval_sites(cb_ctx* c, int snapshot_in, int n_ops, const int32_t* nodes, const int32_t* children,
+                             const int32_t* pslots, const double* pi, int flags, int* snapshot_out, double* lnl_out,
+                             double* site_lnl_out, double* cat_post_out) {
+  return guarded([&] {
+    REQUIRE(c && c->n_states > 0, "cb_set_tips must come first");
+    REQUIRE(site_lnl_out, "null argument: site_lnl_out");
+    REQUIRE(!(flags & CB_EVAL_NO_SYNC), "cb_eval_sites returns its arrays when it returns: CB_EVAL_NO_SYNC is not accepted");
+    CU(cudaSetDevice(c->device));
+    if (!c->d_site_lnl && dev_alloc(c, (void**)&c->d_site_lnl, (size_t)c->P * 8)) return 1;
+    if (cat_post_out && !c->d_site_post && dev_alloc(c, (void**)&c->d_site_post, (size_t)c->n_cats * c->P * 8)) return 1;
+    const int32_t offsets[2] = {0, n_ops};
+    if (eval_impl(c, snapshot_in, 1, offsets, nodes, children, pslots, pi, flags, snapshot_out, lnl_out, c->d_site_lnl,
+                  cat_post_out ? c->d_site_post : nullptr))
+      return 1;
+    // the evaluation has synchronised; the real sites of each row, without the padding
+    const size_t row = (size_t)c->n_sites * 8;
+    CU(cudaMemcpyAsync(site_lnl_out, c->d_site_lnl, row, cudaMemcpyDeviceToHost, c->stream));
+    for (int q = 0; cat_post_out && q < c->n_cats; ++q)
+      CU(cudaMemcpyAsync(cat_post_out + (size_t)q * c->n_sites, c->d_site_post + (size_t)q * c->P, row,
+                         cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    c->d2h += (int64_t)row * (cat_post_out ? 1 + c->n_cats : 1);
+    // The epilogue wrote the category terms t_c it added into s_p; their share of s_p is the posterior.  Dividing here
+    // rather than in the kernel keeps C double divisions out of the root branch of the hot kernels (measured on C4:
+    // the in-kernel form cost the plain evaluation ~0.8 %).  s_p is re-added in the epilogue's order and IEEE division
+    // is correctly rounded on both sides, so q has the bits the epilogue would have produced.
+    if (cat_post_out) {
+      const int64_t n = c->n_sites;
+      for (int64_t p = 0; p < n; ++p) {
+        double s = 0.0;
+        for (int q = 0; q < c->n_cats; ++q) s += cat_post_out[q * n + p];
+        for (int q = 0; q < c->n_cats; ++q) cat_post_out[q * n + p] /= s;
+      }
+    }
+    return 0;
+  });
 }
 
 extern "C" int cb_result_wait(cb_ctx* c, double* lnl_out) {
@@ -1684,6 +1732,13 @@ extern "C" int cb_chain_counters(cb_chain* c, int64_t* moves7, int64_t* accepts7
   memcpy(moves7, c->ch.n_moves, sizeof c->ch.n_moves);
   memcpy(accepts7, c->ch.n_accepts, sizeof c->ch.n_accepts);
   return 0;
+}
+extern "C" int cb_chain_site_lnl(cb_chain* c, double* site_lnl_out, double* cat_post_out) {
+  return guarded([&] {
+    REQUIRE(c && site_lnl_out, "null argument");
+    REQUIRE(c->ch.snap >= 0, "cb_chain_set_state must come first");
+    return chain_err(c, cbm::site_lnl(&c->ch, site_lnl_out, cat_post_out));
+  });
 }
 extern "C" int cb_chain_destroy(cb_chain* c) {
   if (!c) return 0;

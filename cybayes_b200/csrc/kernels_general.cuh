@@ -187,6 +187,8 @@ __global__ void __launch_bounds__(GEN_THREADS) prune_general_kernel(const Launch
 }
 
 // lnL = sum_p w_p * log( sum_c pi.L_root,c / n_cats ), categories brought to a common exponent.
+// With k.site_lnl (cb_eval_sites, single evaluation) every padded site also writes its term, and with k.site_post the
+// category terms added into s (the library divides them by s).
 __global__ void __launch_bounds__(256) root_combine_kernel(const LaunchConst k) {
   __shared__ double red[32];
   __shared__ int last_flag;
@@ -196,7 +198,7 @@ __global__ void __launch_bounds__(256) root_combine_kernel(const LaunchConst k) 
   double lnl = 0.0;
   if (site < P) {
     const double w = __ldcg(k.weights + site);
-    if (w != 0.0) {
+    if (w != 0.0 || k.site_lnl != nullptr) {
       const int64_t base = (int64_t)out * k.n_cats * P + site;
       int emax = INT_MIN;
       for (int c = 0; c < k.n_cats; ++c) emax = max(emax, __ldcg(k.root_exp + base + (int64_t)c * P));
@@ -206,7 +208,16 @@ __global__ void __launch_bounds__(256) root_combine_kernel(const LaunchConst k) 
         const int e = __ldcg(k.root_exp + base + (int64_t)c * P);
         s += ldexp(d, e - emax) / k.cats;
       }
-      lnl = w * (log(s) + (double)emax * 0.693147180559945309417232121458);
+      const double ell = log(s) + (double)emax * 0.693147180559945309417232121458;
+      if (w != 0.0) lnl = w * ell;
+      if (k.site_lnl != nullptr) {
+        k.site_lnl[site] = ell;
+        for (int c = 0; k.site_post != nullptr && c < k.n_cats; ++c) {
+          const double d = __ldcg(k.root_dot + base + (int64_t)c * P);
+          const int e = __ldcg(k.root_exp + base + (int64_t)c * P);
+          k.site_post[(int64_t)c * P + site] = ldexp(d, e - emax) / k.cats;
+        }
+      }
     }
   }
   block_reduce_to_result(lnl, k, out, red, &last_flag);

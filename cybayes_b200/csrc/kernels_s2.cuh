@@ -468,8 +468,14 @@ __global__ void __launch_bounds__(THREADS, MINB) prune_s2_kernel(const LaunchCon
         for (int v = 0; v < V; ++v) {
           double s = 0.0;
 #pragma unroll
-          for (int c = 0; c < C; ++c) s += fma(pi1, out[c][1].v[v], pi0 * out[c][0].v[v]) / k.cats;
-          if (w.v[v] != 0.0) lnl += w.v[v] * (log(s) + (double)e_in[v] * ln2);
+          for (int c = 0; c < C; ++c) {
+            const double t = fma(pi1, out[c][1].v[v], pi0 * out[c][0].v[v]) / k.cats;
+            s += t;
+            if (k.site_post != nullptr) k.site_post[c * P + site + v] = t;   // cb_eval_sites (the library divides by s)
+          }
+          const double ell = log(s) + (double)e_in[v] * ln2;
+          if (w.v[v] != 0.0) lnl += w.v[v] * ell;
+          if (k.site_lnl != nullptr) k.site_lnl[site + v] = ell;   // cb_eval_sites: every padded site, pads included
         }
       }
     }

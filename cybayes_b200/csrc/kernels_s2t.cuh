@@ -557,10 +557,17 @@ __global__ void __launch_bounds__(S2T_THREADS / V, MINB) prune_s2t_kernel(const 
 #pragma unroll
         for (int v = 0; v < V; ++v) {
           const double w = __ldg(k.weights + site + v * S2T_W);
+          const int64_t p = site + v * S2T_W;
           double s = 0.0;
 #pragma unroll
-          for (int c = 0; c < C; ++c) s += fma(pi1, out[v][c][1], pi0 * out[v][c][0]) / k.cats;
-          if (w != 0.0) lnl += w * (log(s) + (double)e_in[v] * ln2);
+          for (int c = 0; c < C; ++c) {
+            const double t = fma(pi1, out[v][c][1], pi0 * out[v][c][0]) / k.cats;
+            s += t;
+            if (k.site_post != nullptr) k.site_post[c * k.n_sites + p] = t;   // cb_eval_sites (the library divides by s)
+          }
+          const double ell = log(s) + (double)e_in[v] * ln2;
+          if (w != 0.0) lnl += w * ell;
+          if (k.site_lnl != nullptr) k.site_lnl[p] = ell;   // cb_eval_sites: every padded site, pads included
 #pragma unroll
           for (int c = 0; c < C; ++c) {   // an (optionally) stored root partial is kept as computed, exponent e_in
             cur[v][c][0] = out[v][c][0];

@@ -122,6 +122,15 @@ static int be_eval(Chain* ch, int snap_in, int n_ops, const int32_t* nodes, cons
   if (ch->be.eval) return ch->be.eval(ch->be.user, snap_in, n_ops, nodes, children, pslots, pi, flags, snap_out, lnl);
   return cb_eval(ch->ctx, snap_in, n_ops, nodes, children, pslots, pi, flags, snap_out, lnl);
 }
+static int be_eval_sites(Chain* ch, int snap_in, int n_ops, const int32_t* nodes, const int32_t* children,
+                         const int32_t* pslots, const double* pi, double* lnl, double* site_lnl, double* cat_post) {
+  int snap_out = -1;
+  if (ch->be.eval_sites)
+    return ch->be.eval_sites(ch->be.user, snap_in, n_ops, nodes, children, pslots, pi, 0, &snap_out, lnl, site_lnl, cat_post);
+  if (ch->be.eval || !ch->ctx)
+    return chain_fail(ch, "native chain: per-site terms need an eval_sites callback when evaluation goes through callbacks");
+  return cb_eval_sites(ch->ctx, snap_in, n_ops, nodes, children, pslots, pi, 0, &snap_out, lnl, site_lnl, cat_post);
+}
 static void be_release(Chain* ch, int snap) {
   if (snap < 0) return;
   if (ch->be.snapshot_release) ch->be.snapshot_release(ch->be.user, snap);
@@ -183,10 +192,9 @@ static inline void op_children(const std::vector<int32_t>& k0, const std::vector
   c_second = k0[node];
 }
 
-// Evaluate the op list of `todo` nodes (in plan order) on `tree`; snap_in < 0 = full evaluation.
-static int evaluate(Chain* ch, const std::vector<Edge>& tree, const std::vector<int32_t>& k0, const std::vector<int32_t>& k1,
-                    const std::vector<int32_t>& todo, int snap_in, const double* pi, int* snap_out, double* lnl,
-                    bool keep_cache = true) {
+// The op list of `todo` nodes (in plan order) on `tree` into ch->nodes / children / pslots.
+static void fill_ops(Chain* ch, const std::vector<Edge>& tree, const std::vector<int32_t>& k0, const std::vector<int32_t>& k1,
+                     const std::vector<int32_t>& todo) {
   const int C = ch->C, n = (int)todo.size();
   ch->nodes.resize(n);
   ch->children.resize(2 * (size_t)n);
@@ -206,7 +214,23 @@ static int evaluate(Chain* ch, const std::vector<Edge>& tree, const std::vector<
       for (int q = 0; q < C; ++q) ch->pslots[(size_t)(2 * i + kx) * C + q] = e.slot[q];
     }
   }
-  return be_eval(ch, snap_in, n, ch->nodes.data(), ch->children.data(), ch->pslots.data(), pi, snap_out, lnl, keep_cache);
+}
+// Evaluate the op list of `todo` nodes (in plan order) on `tree`; snap_in < 0 = full evaluation.
+static int evaluate(Chain* ch, const std::vector<Edge>& tree, const std::vector<int32_t>& k0, const std::vector<int32_t>& k1,
+                    const std::vector<int32_t>& todo, int snap_in, const double* pi, int* snap_out, double* lnl,
+                    bool keep_cache = true) {
+  fill_ops(ch, tree, k0, k1, todo);
+  return be_eval(ch, snap_in, (int)todo.size(), ch->nodes.data(), ch->children.data(), ch->pslots.data(), pi, snap_out, lnl,
+                 keep_cache);
+}
+// Per-site terms of the current state: the root op alone against the chain's snapshot (cb_chain_site_lnl).
+static int site_lnl(Chain* ch, double* out, double* cat_post) {
+  std::vector<int32_t> k0, k1, par;
+  build_kids(ch, ch->tree, k0, k1, par);
+  fill_ops(ch, ch->tree, k0, k1, std::vector<int32_t>{ch->root});
+  double lnl = 0.0;
+  return be_eval_sites(ch, ch->snap, 1, ch->nodes.data(), ch->children.data(), ch->pslots.data(), ch->pi.data(), &lnl, out,
+                       cat_post);
 }
 
 // likelihood first, cache on acceptance?  Only where keeping the cache costs real bandwidth (a cache of 1 GB and more:

@@ -107,10 +107,28 @@ def spr_tables(tmats, tree_prop, pi, rates, site_rates):
     return out
 
 
+def open_site_lnl(output_file, n_columns):
+    """<output_file>.sitelnl with its header: Iter, then the alignment columns 1..n_columns."""
+    fh = open(output_file + ".sitelnl", "w")
+    print("Iter", *range(1, n_columns + 1), sep="\t", file=fh)
+    return fh
+
+
+def write_site_lnl(fh, n_iter, site_lnl):
+    """One sample: the generation, then the log-likelihood of every alignment column (%.17g: round-trips)."""
+    fh.write(str(n_iter) + "\t" + "\t".join(["%.17g" % x for x in site_lnl.tolist()]) + "\n")
+
+
 def run_chain(input_file, model, n_gen, thin, data_type, output_file, reader=None, seed=1234,
-              out=sys.stdout, fast_spr=False, on_generation=None, diag=None, skip_degenerate_rates=False):
+              out=sys.stdout, fast_spr=False, on_generation=None, diag=None, skip_degenerate_rates=False,
+              site_lnl=False):
     """Run the chain; returns a dict with the final state, counters and timings.  `diag` (a dict) receives, before
-    each on_generation call, the acceptance test's two sides: diag["ll_ratio"] and diag["log_u"]."""
+    each on_generation call, the acceptance test's two sides: diag["ll_ratio"] and diag["log_u"].  site_lnl: also
+    write <output_file>.sitelnl, one row of per-column log-likelihoods per sample (the generations of .log), computed
+    from the current cache without a random draw."""
+    if site_lnl:
+        from .likelihood import refuse_sharded_site_lnl
+        refuse_sharded_site_lnl()
     np.random.seed(seed)
     random.seed(seed)
     load_alignment(input_file, data_type, reader)
@@ -142,6 +160,9 @@ def run_chain(input_file, model, n_gen, thin, data_type, output_file, reader=Non
     log_fh = open(output_file + ".log", "w")
     trees_fh = open(output_file + ".trees", "w")
     print("Iter", "LnL", "TL", "Alpha", sep="\t", file=log_fh)
+    site_fh = open_site_lnl(output_file, n_sites) if site_lnl else None
+    if site_fh is not None:
+        from .likelihood import site_log_likelihoods
 
     # np.random.choice(a, p=w) == a[cdf.searchsorted(random_sample(), 'right')] and np.random.choice(a) ==
     # a[randint(0, len(a))] draw for draw (legacy RandomState); the direct forms skip ~35 us of argument checks
@@ -269,9 +290,14 @@ def run_chain(input_file, model, n_gen, thin, data_type, output_file, reader=Non
             print(n_iter, current_ll, proposed_ll, TL, param, name, sep="\t", file=out)
             print(n_iter, state["logLikehood"], TL, state["srates"], sep="\t", file=log_fh)
             print(n_iter, sampled, sep="\t", file=trees_fh)
+            if site_fh is not None:
+                write_site_lnl(site_fh, n_iter, site_log_likelihoods(state["pi"], root, leaves, state["postorder"],
+                                                                     state["transitionMat"], cache=cache)[1])
     elapsed = time.perf_counter() - t_start
     log_fh.close()
     trees_fh.close()
+    if site_fh is not None:
+        site_fh.close()
     for k, v in moves_count.items():
         print(k, accepts_count[k], v, file=out)
     return {"state": state, "initial_lnL": initial_lnl, "moves": dict(moves_count), "accepts": dict(accepts_count),
@@ -291,14 +317,22 @@ def main(argv=None):
     ap.add_argument("--native", action="store_true", help="run the generation loop inside the library (same trace)")
     ap.add_argument("--skip-degenerate-rates", action="store_true",
                     help="GTR on binary data: do not propose the single exchangeability (the reference crashes there)")
+    ap.add_argument("--site-lnl", action="store_true",
+                    help="also write <output>.sitelnl: per-column log-likelihoods at every sample (WAIC / LOO input)")
     a = ap.parse_args(argv)
+    if a.site_lnl:
+        from .likelihood import refuse_sharded_site_lnl
+        try:
+            refuse_sharded_site_lnl()
+        except ValueError as e:
+            ap.error(f"--site-lnl: {e}")
     if a.native:
         from .fastchain import run_chain_native
         res = run_chain_native(a.input_file, a.model, a.n_gen, a.thin, a.data_type, a.output_file, reader=a.reader,
-                               skip_degenerate_rates=a.skip_degenerate_rates)
+                               skip_degenerate_rates=a.skip_degenerate_rates, site_lnl=a.site_lnl)
     else:
         res = run_chain(a.input_file, a.model, a.n_gen, a.thin, a.data_type, a.output_file, reader=a.reader,
-                        fast_spr=a.fast_spr, skip_degenerate_rates=a.skip_degenerate_rates)
+                        fast_spr=a.fast_spr, skip_degenerate_rates=a.skip_degenerate_rates, site_lnl=a.site_lnl)
     print(f"# {res['gens_per_sec']:.1f} generations/s", file=sys.stderr)
 
 

@@ -179,6 +179,21 @@ class Engine(SlotPool):
                                 _f64(self._lnl)))
         return float(self._lnl[0]), int(self._snap.value)
 
+    def eval_sites(self, snapshot, nodes, children, pslots, pi, want_snapshot=False, categories=False,
+                   force_levels=False, force_walk=False, no_fold=False):
+        """cb_eval with the per-pattern terms of lnL (see cb_eval_sites).  Returns (lnL, site_lnl[n_patterns],
+        post[n_cats, n_patterns] -- the rate-category posteriors -- or None, snapshot id or -1)."""
+        self.flush_builds()
+        flags = (CB_EVAL_WANT_SNAPSHOT if want_snapshot else 0) | (CB_EVAL_FORCE_LEVELS if force_levels else 0) \
+            | (CB_EVAL_FORCE_WALK if force_walk else 0) | (CB_EVAL_NO_FOLD if no_fold else 0)
+        pi = np.ascontiguousarray(pi, dtype=np.float64)
+        site = np.empty(self.n_patterns)
+        post = np.empty((self.n_cats, self.n_patterns)) if categories else None
+        check(self._lib.cb_eval_sites(self._ctx, -1 if snapshot is None else int(snapshot), nodes.size, _i32(nodes),
+                                      _i32(children), _i32(pslots), _f64(pi), flags, C.byref(self._snap),
+                                      _f64(self._lnl), _f64(site), None if post is None else _f64(post)))
+        return float(self._lnl[0]), site, post, int(self._snap.value)
+
     def eval_batch(self, snapshot, offsets, nodes, children, pslots, pi):
         """Score many candidate dirty paths against one snapshot in a single launch."""
         self.flush_builds()

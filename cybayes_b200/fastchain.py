@@ -21,7 +21,7 @@ import numpy as np
 
 from . import _lib, config, likelihood, subst
 from ._lib import c_f64p, c_i32p
-from .driver import load_alignment, move_table
+from .driver import load_alignment, move_table, open_site_lnl, write_site_lnl
 from .mcmc_gamma import adjlist2newickBL, adjlist2nodes_dict, get_siterates, state_init
 
 MOVES = [("bl", "scale_edge"), ("bl", "node_slider"), ("tree", "rooted_NNI"), ("tree", "externalSPR"),
@@ -31,6 +31,7 @@ MODEL_IDS = {"JC": 0, "F81": 1, "GTR": 2}
 
 _BUILD_FN, _EVAL_FN, _RELEASE_FN = _lib.CHAIN_BUILD_FN, _lib.CHAIN_EVAL_FN, _lib.CHAIN_RELEASE_FN
 _RATES_FN, _BETA_FN, _EIG_FN = _lib.CHAIN_RATES_FN, _lib.CHAIN_BETA_FN, _lib.CHAIN_EIG_FN
+_EVAL_SITES_FN = _lib.CHAIN_EVAL_SITES_FN
 ChainBackend = _lib.ChainBackend
 
 
@@ -65,7 +66,7 @@ def _host_callbacks(n_states, n_cats, n_rates):
 
 def engine_callbacks(engine):
     """Evaluation backend over any object with the Engine methods (the CPU tests pass the oracle-backed fake):
-    (pmat_build, eval, snapshot_release) as ctypes callbacks."""
+    (pmat_build, eval, snapshot_release, eval_sites) as ctypes callbacks."""
     S, Cc = engine.n_states, engine.n_cats
 
     def build_cb(_user, model, pi, beta, gtr, count, slots, d, x):
@@ -98,15 +99,35 @@ def engine_callbacks(engine):
     def release_cb(_user, snap):
         engine.release_snapshot(snap)
         return 0
-    return _BUILD_FN(build_cb), _EVAL_FN(eval_cb), _RELEASE_FN(release_cb)
+
+    def eval_sites_cb(_user, snap_in, n_ops, nodes, children, pslots, pi, flags, snap_out, lnl_out, site_out, post_out):
+        try:
+            lnl, site, post, snap = engine.eval_sites(
+                None if snap_in < 0 else snap_in, np.ctypeslib.as_array(nodes, shape=(n_ops,)).copy(),
+                np.ctypeslib.as_array(children, shape=(2 * n_ops,)).copy(),
+                np.ctypeslib.as_array(pslots, shape=(2 * n_ops, Cc)).copy(), np.ctypeslib.as_array(pi, shape=(S,)).copy(),
+                want_snapshot=bool(flags & 1), categories=bool(post_out))
+            P = engine.n_patterns
+            np.ctypeslib.as_array(site_out, shape=(P,))[:] = site
+            if post_out:
+                np.ctypeslib.as_array(post_out, shape=(Cc, P))[:] = post
+            snap_out[0] = snap
+            lnl_out[0] = lnl
+            return 0
+        except Exception:
+            import traceback
+            traceback.print_exc()
+            return 1
+    return _BUILD_FN(build_cb), _EVAL_FN(eval_cb), _RELEASE_FN(release_cb), _EVAL_SITES_FN(eval_sites_cb)
 
 
 class NativeChain:
     """Thin object over cb_chain_*; the start state comes from Python, generations run in the library."""
 
-    def __init__(self, engine, state, site_rates, model, binary, use_callbacks=False, skip_degenerate_rates=False):
+    def __init__(self, engine, state, site_rates, model, binary, use_callbacks=False, skip_degenerate_rates=False,
+                 site_map=None):
         lib = _lib.load()
-        self._lib, self.engine = lib, engine
+        self._lib, self.engine, self._site_map = lib, engine, site_map
         self.n_taxa, self.n_states, self.n_cats = config.N_TAXA, engine.n_states, engine.n_cats
         tree = state["tree"]
         self.n_edges = len(tree)
@@ -122,7 +143,7 @@ class NativeChain:
         ctx = None
         if use_callbacks or not hasattr(engine, "_ctx") or not isinstance(engine._ctx, C.c_void_p):
             self._eng_cbs = engine_callbacks(engine)
-            be.pmat_build, be.eval, be.snapshot_release = self._eng_cbs
+            be.pmat_build, be.eval, be.snapshot_release, be.eval_sites = self._eng_cbs
         else:
             engine.flush_builds()
             ctx = engine._ctx
@@ -199,6 +220,20 @@ class NativeChain:
         return {"tree": tree, "pi": pi, "rates": rates, "srates": alpha.value, "site_rates": sr.tolist(),
                 "logLikehood": np.float64(lnl.value)}
 
+    def site_lnl(self, categories=False):
+        """Per-column terms of the current state's lnL (cb_chain_site_lnl), in alignment-column order when the engine
+        holds compressed patterns (`site_map`), and with categories the (n_cats, columns) rate-category posteriors.
+        Returns (site_lnl, post or None).  Takes no random draw."""
+        P = self.engine.n_patterns
+        site = np.empty(P)
+        post = np.empty((self.n_cats, P)) if categories else None
+        _lib.check(self._lib.cb_chain_site_lnl(self._chain, site.ctypes.data_as(c_f64p),
+                                               None if post is None else post.ctypes.data_as(c_f64p)))
+        if self._site_map is not None:
+            site = site[self._site_map]
+            post = None if post is None else post[:, self._site_map]
+        return site, post
+
     def counters(self):
         m, a = np.zeros(7, dtype=np.int64), np.zeros(7, dtype=np.int64)
         i64p = C.POINTER(C.c_int64)
@@ -219,8 +254,11 @@ class NativeChain:
 
 
 def run_chain_native(input_file, model, n_gen, thin, data_type, output_file, reader=None, seed=1234, out=sys.stdout,
-                     on_generation=None, diag=None, use_callbacks=False, skip_degenerate_rates=False):
-    """driver.run_chain with the generation loop in the library; same files, same stdout, same return value."""
+                     on_generation=None, diag=None, use_callbacks=False, skip_degenerate_rates=False, site_lnl=False):
+    """driver.run_chain with the generation loop in the library; same files, same stdout, same return value.
+    site_lnl: also write <output_file>.sitelnl (driver.run_chain), from cb_chain_site_lnl at every sample."""
+    if site_lnl:
+        likelihood.refuse_sharded_site_lnl()
     np.random.seed(seed)
     random.seed(seed)
     load_alignment(input_file, data_type, reader)
@@ -234,9 +272,9 @@ def run_chain_native(input_file, model, n_gen, thin, data_type, output_file, rea
     state = state_init()
     site_rates = get_siterates(state["srates"])
     root = state["root"]
-    engine, _ = likelihood.engine_for(config.LEAF_LLMAT, config.N_CATS)
+    engine, site_map = likelihood.engine_for(config.LEAF_LLMAT, config.N_CATS)
     chain = NativeChain(engine, state, site_rates, model, config.IN_DTYPE == "bin", use_callbacks=use_callbacks,
-                        skip_degenerate_rates=skip_degenerate_rates)
+                        skip_degenerate_rates=skip_degenerate_rates, site_map=site_map)
     state["logLikehood"] = np.float64(chain.initial_lnl)
     print("Initial Random Tree ", adjlist2newickBL(state["tree"], adjlist2nodes_dict(state["tree"]), root) + ";",
           sep="\t", file=out)
@@ -245,6 +283,7 @@ def run_chain_native(input_file, model, n_gen, thin, data_type, output_file, rea
     log_fh = open(output_file + ".log", "w")
     trees_fh = open(output_file + ".trees", "w")
     print("Iter", "LnL", "TL", "Alpha", sep="\t", file=log_fh)
+    site_fh = open_site_lnl(output_file, config.N_SITES) if site_lnl else None
     chain.take_rng()
     first_seen = {}
     want_trace = True
@@ -270,10 +309,14 @@ def run_chain_native(input_file, model, n_gen, thin, data_type, output_file, rea
             print(done, np.float64(cur[-1]), np.float64(prop[-1]), TL, p, name, sep="\t", file=out)
             print(done, st["logLikehood"], TL, st["srates"], sep="\t", file=log_fh)
             print(done, sampled, sep="\t", file=trees_fh)
+            if site_fh is not None:
+                write_site_lnl(site_fh, done, chain.site_lnl()[0])
     elapsed = time.perf_counter() - t_start
     chain.give_rng()
     log_fh.close()
     trees_fh.close()
+    if site_fh is not None:
+        site_fh.close()
     final = chain.state()
     final["root"] = root
     m, a = chain.counters()

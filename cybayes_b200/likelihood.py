@@ -112,6 +112,13 @@ def _shard_rank():
     return int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))
 
 
+def refuse_sharded_site_lnl():
+    """Per-column log-likelihoods need every pattern and the column -> pattern map; a site-sharded rank has neither."""
+    if os.environ.get("CYBAYES_SHARD", "0") == "1":
+        raise ValueError("per-site log-likelihoods are not available with CYBAYES_SHARD=1: each rank holds only its "
+                         "slice of the patterns (Engine.eval_sites returns that slice)")
+
+
 _comm_serial = 0          # sharded contexts created by this process; never reset (reset_engines included)
 _PROCESS_START = None
 
@@ -510,6 +517,34 @@ def _dirty(pi, root, ll_mats, cache, nodes_recompute, edges, tmats, n_cats_table
     lnl, snap = engine.eval(cache.snap, nodes, children, pslots, np.asarray(pi, dtype=np.float64),
                             want_snapshot=True, store_root=STORE_ROOT)
     return np.float64(lnl), PartialCache(engine, snap, site_map, cache.nodes())
+
+
+def site_log_likelihoods(pi, root, ll_mats, edges, tmats, cache=None, categories=False):
+    """Extension (no reference entry point): the per-column terms of lnL, for site-wise model comparison (WAIC,
+    PSIS-LOO), site-rate estimates and site-wise tree tests.  Returns (lnL, site_lnl[n_columns], post or None) where
+    lnL = sum(site_lnl) and, with categories, post[k, column] is the posterior probability of rate category k (equal
+    category priors).  Arguments as for matML; with the PartialCache of this state only the root is recomputed (a
+    LazyPartialCache not yet materialised, or no cache: one full pass that keeps nothing)."""
+    refuse_sharded_site_lnl()
+    engine, site_map = engine_for(ll_mats, len(tmats))
+    plan = _plan_for(edges)
+    if plan.nodes[-1] != root:
+        raise KeyError(root)
+    pi = np.asarray(pi, dtype=np.float64)
+    if cache is not None and (not isinstance(cache, PartialCache) or cache.engine is not engine):
+        raise TypeError("cache must be the cache returned by matML/cache_matML for this alignment")
+    if cache is not None and not (isinstance(cache, LazyPartialCache) and cache._snap is None):
+        kids = plan.kids[root]
+        pslots, keep = _slot_matrix(engine, tmats, [(root, c) for c in kids])
+        lnl, site, post, _ = engine.eval_sites(cache.snap, np.array([root], dtype=np.int32),
+                                               np.array(kids, dtype=np.int32), pslots, pi, categories=categories)
+    else:
+        pslots, keep = _slot_matrix(engine, tmats, plan.edge_keys, plan=plan)
+        lnl, site, post, _ = engine.eval_sites(None, plan.nodes, plan.children, pslots, pi, categories=categories)
+    if site_map is not None:
+        site = site[site_map]
+        post = None if post is None else post[:, site_map]
+    return np.float64(lnl), site, post
 
 
 # --------------------------------------------------------- ML_gamma.pyx surface (Gamma rates)

@@ -122,6 +122,19 @@ int cb_eval_batch(cb_ctx* ctx, int snapshot_in, int n_batch, const int32_t* op_o
                   const int32_t* nodes, const int32_t* children, const int32_t* pslots,
                   const double* pi, double* lnl_out);
 int cb_result_wait(cb_ctx* ctx, double* lnl_out);
+/* cb_eval (same op lists, snapshots and flags; CB_EVAL_NO_SYNC is rejected) that also returns the per-site terms of
+ * lnL, for site-wise model comparison (WAIC, PSIS-LOO), site-rate estimates and site-wise tree tests.  For pattern p
+ * of the context (n_sites = the count given to cb_set_tips: on a sharded context the rank's own slice), with the
+ * root partial L_c,p kept as mantissas and one exponent e_p (a power of two, common to the categories):
+ *   s_p = sum_c pi . L_c,p / n_cats
+ *   site_lnl_out[p]          = log(s_p) + e_p ln 2            (lnL = sum_p w_p site_lnl_out[p], the very terms summed)
+ *   cat_post_out[c][p]       = (pi . L_c,p / n_cats) / s_p    (posterior of rate category c, equal priors)
+ * cat_post_out may be NULL.  lnl_out equals cb_eval's bit for bit (the same launches and reduction; on a sharded
+ * context the all-reduced total).  The root kernel writes l and the category terms, which are copied back once;
+ * q is their share of s_p, divided on the host. */
+int cb_eval_sites(cb_ctx* ctx, int snapshot_in, int n_ops, const int32_t* nodes, const int32_t* children,
+                  const int32_t* pslots, const double* pi, int flags, int* snapshot_out, double* lnl_out,
+                  double* site_lnl_out /* [n_sites] */, double* cat_post_out /* [n_cats][n_sites] or NULL */);
 
 int cb_snapshot_retain(cb_ctx* ctx, int snapshot);
 int cb_snapshot_release(cb_ctx* ctx, int snapshot);
@@ -136,8 +149,10 @@ int cb_snapshot_read(cb_ctx* ctx, int snapshot, int node, double* out, int32_t* 
  * caller.  For a fixed seed it takes the reference's moves and decisions generation by generation: both random
  * streams (Python `random`, NumPy legacy global generator: MT19937 states handed in and out) and the insertion
  * order of the tree dict are reproduced.  The backend table lets a test replace the CUDA evaluation by callbacks;
- * its last three members are host functions whose bits depend on SciPy / BLAS and are therefore always supplied
- * by the caller (discrete-Gamma rates mcmc_gamma.pyx:596-602, beta = 1/(1 - pi.pi) :467, GTR eigensystem).     */
+ * its three host-maths members are functions whose bits depend on SciPy / BLAS and are therefore always supplied
+ * by the caller (discrete-Gamma rates mcmc_gamma.pyx:596-602, beta = 1/(1 - pi.pi) :467, GTR eigensystem).
+ * eval_sites (cb_eval_sites without the context) serves cb_chain_site_lnl; NULL = the context's own, which a
+ * backend of evaluation callbacks cannot use.                                                                   */
 typedef struct cb_chain cb_chain;
 typedef struct cb_chain_backend {
   void* user;
@@ -151,6 +166,9 @@ typedef struct cb_chain_backend {
   int (*site_rates)(void* user, double alpha, double* rates_out /* n_cats */);
   int (*f81_beta)(void* user, const double* pi, int n_states, double* beta_out);
   int (*gtr_eig)(void* user, const double* pi, const double* exchangeabilities, double* eig_out /* S + 2 S S */);
+  int (*eval_sites)(void* user, int snapshot_in, int n_ops, const int32_t* nodes, const int32_t* children,
+                    const int32_t* pslots, const double* pi, int flags, int* snapshot_out, double* lnl_out,
+                    double* site_lnl_out, double* cat_post_out);
 } cb_chain_backend;
 /* model: 0 JC, 1 F81, 2 GTR.  param_ids[n_params] in the driver's order (0 pi, 1 rates, 2 tree, 3 bl, 4 srates)
  * with their cumulative normalised weights; tree_cdf[2] = (NNI, eSPR), bl_cdf[2] = (scale_edge, node_slider)
@@ -174,6 +192,10 @@ int cb_chain_run(cb_chain* chain, int64_t n_gens, int8_t* move, int8_t* accepted
 int cb_chain_get_state(cb_chain* chain, int32_t* parents, int32_t* children, double* lengths, double* pi,
                        double* rates, double* alpha, double* site_rates, double* lnl);
 int cb_chain_counters(cb_chain* chain, int64_t* moves7, int64_t* accepts7);
+/* Per-site terms of the chain's current state (see cb_eval_sites): one root-only evaluation against the chain's
+ * snapshot with its current P matrices and pi.  Between cb_chain_run calls; leaves the chain's random streams,
+ * counters, state and snapshot as they are. */
+int cb_chain_site_lnl(cb_chain* chain, double* site_lnl_out, double* cat_post_out);
 int cb_chain_destroy(cb_chain* chain);
 
 /* ---- introspection / measurement ---------------------------------------------------------- */
