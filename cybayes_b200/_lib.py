@@ -67,6 +67,8 @@ SIGNATURES = {
     "cb_eval_sites": (C.c_int, [C.c_void_p, C.c_int, C.c_int, c_i32p, c_i32p, c_i32p, c_f64p, C.c_int,
                                 C.POINTER(C.c_int), c_f64p, c_f64p, c_f64p]),
     "cb_eval_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_int, c_i32p, c_i32p, c_i32p, c_i32p, c_f64p, c_f64p]),
+    "cb_simulate": (C.c_int, [C.c_void_p, C.c_int, c_i32p, c_i32p, c_i32p, c_f64p, C.c_int, C.c_uint64, C.c_uint32,
+                              C.c_int64, C.c_void_p]),
     "cb_result_wait": (C.c_int, [C.c_void_p, c_f64p]),
     "cb_snapshot_retain": (C.c_int, [C.c_void_p, C.c_int]),
     "cb_snapshot_release": (C.c_int, [C.c_void_p, C.c_int]),

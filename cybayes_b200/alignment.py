@@ -222,6 +222,14 @@ def compress_patterns_gpu(codes, device=None):
     """compress_patterns for alignments too long for the host route (10^5 .. 10^7 columns): the column comparison runs
     on the GPU (cb_compress_patterns: 128-bit column hashes, verified column by column, so the result is exact).
     Same return value as compress_patterns, element for element."""
+    codes = np.ascontiguousarray(codes)
+    weights, site_to_pattern, first = pattern_weights_gpu(codes, device)
+    return np.ascontiguousarray(codes[:, first]), weights, site_to_pattern
+
+
+def pattern_weights_gpu(codes, device=None):
+    """compress_patterns_gpu without gathering the pattern columns: (weights, site_to_pattern, first_site) -- what a
+    statistic of the column multiplicities needs."""
     import ctypes as C
 
     from . import _lib
@@ -238,4 +246,4 @@ def compress_patterns_gpu(codes, device=None):
                                         site_to_pattern.ctypes.data_as(_lib.c_i64p), first.ctypes.data_as(_lib.c_i64p),
                                         weights.ctypes.data_as(_lib.c_f64p), C.byref(n_pat)))
     n = n_pat.value
-    return np.ascontiguousarray(codes[:, first[:n]]), weights[:n].copy(), site_to_pattern
+    return weights[:n].copy(), site_to_pattern, first[:n].copy()

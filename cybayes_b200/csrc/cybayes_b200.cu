@@ -30,6 +30,7 @@
 #include "kernels_pmat.cuh"
 #include "kernels_s2.cuh"
 #include "kernels_s2t.cuh"
+#include "ppc/kernels_sim.cuh"
 
 using namespace cb;
 
@@ -176,6 +177,8 @@ struct cb_ctx {
   int out_cap = 0, max_blocks = 0;
   double* d_site_lnl = nullptr;   // [P], cb_eval_sites only (allocated on first use)
   double* d_site_post = nullptr;  // [C][P], cb_eval_sites with category posteriors only
+  void* d_sim_states = nullptr;   // cb_simulate: internal-node states [n_taxa - 1][n_sites] when they do not fit shared memory
+  size_t sim_states_bytes = 0;
   int last_n_out = 0;
   // scratch for pmat builds
   void* d_scratch = nullptr;
@@ -292,6 +295,8 @@ static int create_impl(int device, cb_ctx** out) {
   CU(cudaFuncSetAttribute(prune_dmma_rc_kernel<SS, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RcCfg<SS>::SMEM))
   CB_RC_ATTR(16); CB_RC_ATTR(24); CB_RC_ATTR(32); CB_RC_ATTR(40); CB_RC_ATTR(48); CB_RC_ATTR(56); CB_RC_ATTR(64);
 #undef CB_RC_ATTR
+  CU(cudaFuncSetAttribute(simulate_kernel<uint8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, SIM_SMEM_MAX));
+  CU(cudaFuncSetAttribute(simulate_kernel<uint16_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, SIM_SMEM_MAX));
   if (const char* v = getenv("CYBAYES_RC_STAGGER")) c->rc_stagger = atoi(v) != 0;
   *out = c;
   return 0;
@@ -337,6 +342,9 @@ static void free_alignment(cb_ctx* c) {
   if (c->d_site_lnl) dev_free(c, c->d_site_lnl, (size_t)c->P * 8);
   if (c->d_site_post) dev_free(c, c->d_site_post, (size_t)c->n_cats * c->P * 8);
   c->d_site_lnl = c->d_site_post = nullptr;
+  if (c->d_sim_states) dev_free(c, c->d_sim_states, c->sim_states_bytes);
+  c->d_sim_states = nullptr;
+  c->sim_states_bytes = 0;
 }
 
 extern "C" int cb_destroy(cb_ctx* c) {
@@ -1352,6 +1360,110 @@ extern "C" int cb_eval_sites(cb_ctx* c, int snapshot_in, int n_ops, const int32_
       }
     }
     return 0;
+  });
+}
+
+// ----------------------------------------------------------------------------- posterior predictive replicates
+static int simulate_impl(cb_ctx* c, int n_edges, const int32_t* parents, const int32_t* children, const int32_t* pslots,
+                         const double* pi, int root, uint64_t seed, uint32_t replicate, int64_t column_offset,
+                         void* codes_out) {
+  REQUIRE(c && c->n_states > 0, "cb_set_tips must come first");
+  REQUIRE(parents && children && pslots && pi, "null argument");
+  const int N = c->n_taxa, S = c->n_states, Cn = c->n_cats, n_nodes = 2 * N - 1;
+  for (size_t s = 0; s < c->snaps.size(); ++s)
+    REQUIRE(c->snaps[s].refs <= 0, "cb_simulate: the context holds live snapshot %d, whose partials would describe the "
+            "old alignment; release every snapshot first", (int)s);
+  REQUIRE(n_edges == 2 * N - 2, "cb_simulate: %d edges, a rooted binary tree of %d taxa has %d", n_edges, N, 2 * N - 2);
+  REQUIRE(root > N && root <= n_nodes, "cb_simulate: root %d is not an internal node (%d..%d)", root, N + 1, n_nodes);
+  REQUIRE(column_offset >= 0 && column_offset <= INT64_MAX - c->n_sites, "cb_simulate: column_offset %lld out of range",
+          (long long)column_offset);
+  for (int i = 0; i < S; ++i) REQUIRE(pi[i] >= 0.0 && pi[i] <= 1.0, "cb_simulate: pi[%d] = %g is not a probability", i, pi[i]);
+  // parents before children: a parent is the root or the child of an earlier edge; every other node is a child once
+  std::vector<char> seen((size_t)n_nodes + 1, 0);
+  seen[root] = 1;
+  const int wi = 2 + Cn, wt = 1 + Cn;
+  std::vector<int32_t> inner, tips((size_t)N * wt, -1);
+  inner.reserve((size_t)(N - 2) * wi);
+  for (int e = 0; e < n_edges; ++e) {
+    const int p = parents[e], ch = children[e];
+    REQUIRE(p > N && p <= n_nodes, "cb_simulate: edge %d: parent %d is not an internal node", e, p);
+    REQUIRE(ch >= 1 && ch <= n_nodes, "cb_simulate: edge %d: child %d is not a node id", e, ch);
+    REQUIRE(seen[p], "cb_simulate: edge %d: parent %d comes before any edge into it (edges must list parents first)", e, p);
+    REQUIRE(!seen[ch], "cb_simulate: edge %d: node %d is the child of a second edge (or the root)", e, ch);
+    seen[ch] = 1;
+    for (int q = 0; q < Cn; ++q)
+      REQUIRE(pslots[(size_t)e * Cn + q] >= 0 && pslots[(size_t)e * Cn + q] < c->pmat_cap,
+              "cb_simulate: P slot %d out of range (reserved %d)", pslots[(size_t)e * Cn + q], c->pmat_cap);
+    int32_t* slots;
+    if (ch <= N) {   // tip row: parent, slots
+      int32_t* row = &tips[(size_t)(ch - 1) * wt];
+      row[0] = p;
+      slots = row + 1;
+    } else {         // inner row: parent, child, slots
+      inner.resize(inner.size() + wi);
+      int32_t* row = &inner[inner.size() - wi];
+      row[0] = p;
+      row[1] = ch;
+      slots = row + 2;
+    }
+    memcpy(slots, pslots + (size_t)e * Cn, (size_t)Cn * 4);
+  }
+  const int n_inner = (int)inner.size() / wi;
+  CU(cudaSetDevice(c->device));
+  const bool force_scratch = getenv("CYBAYES_SIM_SCRATCH") && atoi(getenv("CYBAYES_SIM_SCRATCH")) != 0;
+  const size_t smem = (size_t)(N - 1) * SIM_THREADS * c->code_bytes;
+  const bool in_smem = !force_scratch && smem <= (size_t)SIM_SMEM_MAX;
+  if (!in_smem) {
+    const size_t need = (size_t)(N - 1) * c->n_sites * c->code_bytes;
+    if (need > c->sim_states_bytes) {
+      CU(cudaStreamSynchronize(c->stream));
+      if (c->d_sim_states) dev_free(c, c->d_sim_states, c->sim_states_bytes);
+      c->d_sim_states = nullptr;
+      c->sim_states_bytes = 0;
+      if (dev_alloc(c, &c->d_sim_states, need)) return 1;
+      c->sim_states_bytes = need;
+    }
+  }
+  // one upload: pi[S] | inner edges | tip edges
+  const size_t bytes = (size_t)S * 8 + (inner.size() + tips.size()) * 4;
+  if (ensure_scratch(c, bytes)) return 1;
+  CU(cudaEventSynchronize(c->ev_scratch));  // the previous copy out of the pinned scratch has finished
+  unsigned char* h = (unsigned char*)c->h_scratch;
+  memcpy(h, pi, (size_t)S * 8);
+  memcpy(h + (size_t)S * 8, inner.data(), inner.size() * 4);
+  memcpy(h + (size_t)S * 8 + inner.size() * 4, tips.data(), tips.size() * 4);
+  CU(cudaMemcpyAsync(c->d_scratch, c->h_scratch, bytes, cudaMemcpyHostToDevice, c->stream));
+  CU(cudaEventRecord(c->ev_scratch, c->stream));
+  c->h2d += (int64_t)bytes;
+  const unsigned char* d = (const unsigned char*)c->d_scratch;
+  const double* d_pi = (const double*)d;
+  const int32_t* d_inner = (const int32_t*)(d + (size_t)S * 8);
+  const int32_t* d_tips = d_inner + inner.size();
+  const unsigned blocks = (unsigned)((c->n_sites + SIM_THREADS - 1) / SIM_THREADS);
+  const size_t dyn = in_smem ? smem : 0;
+  if (c->code_bytes == 1)
+    simulate_kernel<uint8_t><<<blocks, SIM_THREADS, dyn, c->stream>>>(
+        (uint8_t*)c->d_codes, c->P, c->n_sites, N, S, Cn, n_inner, d_inner, d_tips, c->d_pmats, d_pi, root,
+        (unsigned long long)seed, replicate, (long long)column_offset, in_smem ? nullptr : (uint8_t*)c->d_sim_states);
+  else
+    simulate_kernel<uint16_t><<<blocks, SIM_THREADS, dyn, c->stream>>>(
+        (uint16_t*)c->d_codes, c->P, c->n_sites, N, S, Cn, n_inner, d_inner, d_tips, c->d_pmats, d_pi, root,
+        (unsigned long long)seed, replicate, (long long)column_offset, in_smem ? nullptr : (uint16_t*)c->d_sim_states);
+  CU(cudaGetLastError());
+  c->launches += 1;
+  if (codes_out) {
+    const size_t row = (size_t)c->n_sites * c->code_bytes;
+    CU(cudaMemcpy2DAsync(codes_out, row, c->d_codes, (size_t)c->P * c->code_bytes, row, N, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    c->d2h += (int64_t)row * N;
+  }
+  return 0;
+}
+extern "C" int cb_simulate(cb_ctx* c, int n_edges, const int32_t* parents, const int32_t* children, const int32_t* pslots,
+                           const double* pi, int root, uint64_t seed, uint32_t replicate, int64_t column_offset,
+                           void* codes_out) {
+  return guarded([&] {
+    return simulate_impl(c, n_edges, parents, children, pslots, pi, root, seed, replicate, column_offset, codes_out);
   });
 }
 

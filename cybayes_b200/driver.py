@@ -121,14 +121,18 @@ def write_site_lnl(fh, n_iter, site_lnl):
 
 def run_chain(input_file, model, n_gen, thin, data_type, output_file, reader=None, seed=1234,
               out=sys.stdout, fast_spr=False, on_generation=None, diag=None, skip_degenerate_rates=False,
-              site_lnl=False):
+              site_lnl=False, ppc=0, ppc_seed=1):
     """Run the chain; returns a dict with the final state, counters and timings.  `diag` (a dict) receives, before
     each on_generation call, the acceptance test's two sides: diag["ll_ratio"] and diag["log_u"].  site_lnl: also
     write <output_file>.sitelnl, one row of per-column log-likelihoods per sample (the generations of .log), computed
-    from the current cache without a random draw."""
+    from the current cache without a random draw.  ppc: also write <output_file>.ppc, `ppc` posterior predictive
+    replicates per sample (ppc.write_sample), simulated from Philox streams keyed on ppc_seed: no MT19937 draw."""
     if site_lnl:
         from .likelihood import refuse_sharded_site_lnl
         refuse_sharded_site_lnl()
+    if ppc:
+        from .ppc import refuse_sharded_ppc
+        refuse_sharded_ppc()
     np.random.seed(seed)
     random.seed(seed)
     load_alignment(input_file, data_type, reader)
@@ -163,6 +167,10 @@ def run_chain(input_file, model, n_gen, thin, data_type, output_file, reader=Non
     site_fh = open_site_lnl(output_file, n_sites) if site_lnl else None
     if site_fh is not None:
         from .likelihood import site_log_likelihoods
+    reps = ppc_fh = None
+    if ppc:
+        from .ppc import Replicates, open_ppc, write_sample
+        reps, ppc_fh = Replicates(leaves, n_cats), open_ppc(output_file)
 
     # np.random.choice(a, p=w) == a[cdf.searchsorted(random_sample(), 'right')] and np.random.choice(a) ==
     # a[randint(0, len(a))] draw for draw (legacy RandomState); the direct forms skip ~35 us of argument checks
@@ -293,11 +301,16 @@ def run_chain(input_file, model, n_gen, thin, data_type, output_file, reader=Non
             if site_fh is not None:
                 write_site_lnl(site_fh, n_iter, site_log_likelihoods(state["pi"], root, leaves, state["postorder"],
                                                                      state["transitionMat"], cache=cache)[1])
+            if reps is not None:
+                write_sample(ppc_fh, reps, n_iter, n_iter // thin - 1, state, model, ppc, ppc_seed)
     elapsed = time.perf_counter() - t_start
     log_fh.close()
     trees_fh.close()
     if site_fh is not None:
         site_fh.close()
+    if reps is not None:
+        ppc_fh.close()
+        reps.close()
     for k, v in moves_count.items():
         print(k, accepts_count[k], v, file=out)
     return {"state": state, "initial_lnL": initial_lnl, "moves": dict(moves_count), "accepts": dict(accepts_count),
@@ -319,7 +332,20 @@ def main(argv=None):
                     help="GTR on binary data: do not propose the single exchangeability (the reference crashes there)")
     ap.add_argument("--site-lnl", action="store_true",
                     help="also write <output>.sitelnl: per-column log-likelihoods at every sample (WAIC / LOO input)")
+    ap.add_argument("--ppc", type=int, default=0, metavar="N",
+                    help="also write <output>.ppc: N posterior predictive replicates per sample (lnL and multinomial T)")
+    ap.add_argument("--ppc-seed", type=int, default=1, help="seed of the replicates' Philox streams (0 .. 2^64 - 1)")
     a = ap.parse_args(argv)
+    if a.ppc < 0:
+        ap.error("--ppc: the number of replicates per sample cannot be negative")
+    if not 0 <= a.ppc_seed < 1 << 64:
+        ap.error("--ppc-seed must be in 0 .. 2^64 - 1")
+    if a.ppc:
+        from .ppc import refuse_sharded_ppc
+        try:
+            refuse_sharded_ppc()
+        except ValueError as e:
+            ap.error(f"--ppc: {e}")
     if a.site_lnl:
         from .likelihood import refuse_sharded_site_lnl
         try:
@@ -329,10 +355,12 @@ def main(argv=None):
     if a.native:
         from .fastchain import run_chain_native
         res = run_chain_native(a.input_file, a.model, a.n_gen, a.thin, a.data_type, a.output_file, reader=a.reader,
-                               skip_degenerate_rates=a.skip_degenerate_rates, site_lnl=a.site_lnl)
+                               skip_degenerate_rates=a.skip_degenerate_rates, site_lnl=a.site_lnl, ppc=a.ppc,
+                               ppc_seed=a.ppc_seed)
     else:
         res = run_chain(a.input_file, a.model, a.n_gen, a.thin, a.data_type, a.output_file, reader=a.reader,
-                        fast_spr=a.fast_spr, skip_degenerate_rates=a.skip_degenerate_rates, site_lnl=a.site_lnl)
+                        fast_spr=a.fast_spr, skip_degenerate_rates=a.skip_degenerate_rates, site_lnl=a.site_lnl,
+                        ppc=a.ppc, ppc_seed=a.ppc_seed)
     print(f"# {res['gens_per_sec']:.1f} generations/s", file=sys.stderr)
 
 

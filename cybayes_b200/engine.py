@@ -77,6 +77,7 @@ class Engine(SlotPool):
             raise TypeError("codes must be uint8 or uint16")
         self.n_taxa, self.n_patterns = codes.shape
         self.n_states, self.n_cats = int(n_states), int(n_cats)
+        self.code_dtype = codes.dtype
         if amb_sets is None:
             amb_sets = np.ones((1, n_states))
         amb_sets = np.ascontiguousarray(amb_sets, dtype=np.float64)
@@ -202,6 +203,25 @@ class Engine(SlotPool):
         pi = np.ascontiguousarray(pi, dtype=np.float64)
         check(self._lib.cb_eval_batch(self._ctx, -1 if snapshot is None else int(snapshot), offsets.size - 1,
                                       _i32(offsets), _i32(nodes), _i32(children), _i32(pslots), _f64(pi), _f64(out)))
+        return out
+
+    def simulate(self, parents, children, pslots, pi, root, seed, replicate, column_offset=0, download=True):
+        """cb_simulate: overwrite every state cell of this context's alignment with a draw from the model (edges
+        parents first, pslots[edge, category]).  Returns the replicate's codes (n_taxa, n_patterns), or None without
+        download."""
+        self.flush_builds()
+        parents = np.ascontiguousarray(parents, dtype=np.int32)
+        children = np.ascontiguousarray(children, dtype=np.int32)
+        pslots = np.ascontiguousarray(pslots, dtype=np.int32)
+        pi = np.ascontiguousarray(pi, dtype=np.float64)
+        if not (parents.size == children.size and pslots.shape == (parents.size, self.n_cats) and pi.size == self.n_states):
+            raise ValueError("parents, children, pslots (n_edges, n_cats) and pi (n_states) do not match")
+        if not 0 <= int(replicate) < 1 << 32 or not 0 <= int(seed) < 1 << 64:
+            raise ValueError("replicate must fit 32 bits and seed 64 bits, unsigned")
+        out = np.empty((self.n_taxa, self.n_patterns), dtype=self.code_dtype) if download else None
+        check(self._lib.cb_simulate(self._ctx, parents.size, _i32(parents), _i32(children), _i32(pslots), _f64(pi),
+                                    int(root), int(seed), int(replicate), int(column_offset),
+                                    None if out is None else out.ctypes.data_as(C.c_void_p)))
         return out
 
     def wait(self):

@@ -254,11 +254,15 @@ class NativeChain:
 
 
 def run_chain_native(input_file, model, n_gen, thin, data_type, output_file, reader=None, seed=1234, out=sys.stdout,
-                     on_generation=None, diag=None, use_callbacks=False, skip_degenerate_rates=False, site_lnl=False):
+                     on_generation=None, diag=None, use_callbacks=False, skip_degenerate_rates=False, site_lnl=False, ppc=0, ppc_seed=1):
     """driver.run_chain with the generation loop in the library; same files, same stdout, same return value.
-    site_lnl: also write <output_file>.sitelnl (driver.run_chain), from cb_chain_site_lnl at every sample."""
+    site_lnl: also write <output_file>.sitelnl (driver.run_chain), from cb_chain_site_lnl at every sample.
+    ppc, ppc_seed: also write <output_file>.ppc (driver.run_chain), from NativeChain.state() at every sample."""
     if site_lnl:
         likelihood.refuse_sharded_site_lnl()
+    if ppc:
+        from .ppc import refuse_sharded_ppc
+        refuse_sharded_ppc()
     np.random.seed(seed)
     random.seed(seed)
     load_alignment(input_file, data_type, reader)
@@ -284,6 +288,10 @@ def run_chain_native(input_file, model, n_gen, thin, data_type, output_file, rea
     trees_fh = open(output_file + ".trees", "w")
     print("Iter", "LnL", "TL", "Alpha", sep="\t", file=log_fh)
     site_fh = open_site_lnl(output_file, config.N_SITES) if site_lnl else None
+    reps = ppc_fh = None
+    if ppc:
+        from .ppc import Replicates, open_ppc, write_sample
+        reps, ppc_fh = Replicates(config.LEAF_LLMAT, config.N_CATS), open_ppc(output_file)
     chain.take_rng()
     first_seen = {}
     want_trace = True
@@ -311,12 +319,18 @@ def run_chain_native(input_file, model, n_gen, thin, data_type, output_file, rea
             print(done, sampled, sep="\t", file=trees_fh)
             if site_fh is not None:
                 write_site_lnl(site_fh, done, chain.site_lnl()[0])
+            if reps is not None:
+                st["root"] = root
+                write_sample(ppc_fh, reps, done, done // thin - 1, st, model, ppc, ppc_seed)
     elapsed = time.perf_counter() - t_start
     chain.give_rng()
     log_fh.close()
     trees_fh.close()
     if site_fh is not None:
         site_fh.close()
+    if reps is not None:
+        ppc_fh.close()
+        reps.close()
     final = chain.state()
     final["root"] = root
     m, a = chain.counters()

@@ -136,6 +136,21 @@ int cb_eval_sites(cb_ctx* ctx, int snapshot_in, int n_ops, const int32_t* nodes,
                   const int32_t* pslots, const double* pi, int flags, int* snapshot_out, double* lnl_out,
                   double* site_lnl_out /* [n_sites] */, double* cat_post_out /* [n_cats][n_sites] or NULL */);
 
+/* ---- posterior predictive replicates ------------------------------------------------------
+ * Overwrite, in place, every state cell (code < n_states) of the context's alignment with a draw from the model:
+ * category uniform over n_cats, root from pi, child from P[slot][parent_state][.]. Ambiguity cells and padding are
+ * kept. Edges: parents before children (validated); n_edges = 2 n_taxa - 2, every node but the root the child of one
+ * edge. pslots[e * n_cats + c]. Random numbers: Philox4x32-10 with key (seed lo32, seed hi32) and counter
+ * (k / 4, column lo32, column hi32, replicate), draw k = output word k % 4; k = 0 the category (x * n_cats) >> 32,
+ * k = 1 the root state, k = 1 + child node id the state at that child; a draw is u = (x + 0.5) 2^-32 and picks the
+ * first j with u < row[0] + ... + row[j] (fp64, left to right), else n_states - 1.  Column index = column_offset +
+ * local column, so the slices of a sharded alignment are slices of one replicate. Fails if the context holds a live
+ * snapshot (its partials would describe the old data). codes_out [n_taxa][n_sites] (may be NULL) receives the
+ * replicate. */
+int cb_simulate(cb_ctx* ctx, int n_edges, const int32_t* parents, const int32_t* children, const int32_t* pslots,
+                const double* pi, int root, uint64_t seed, uint32_t replicate, int64_t column_offset,
+                void* codes_out);
+
 int cb_snapshot_retain(cb_ctx* ctx, int snapshot);
 int cb_snapshot_release(cb_ctx* ctx, int snapshot);
 /* out[n_cats][n_states][n_sites] unscaled = stored * 2^scale; scale_out[n_sites] may be NULL,
